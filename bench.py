@@ -26,6 +26,8 @@ collective on the data path).
   tools            the other tools of BASELINE.json's configs, one entry each (N = 1 only):
                    ms per step, arcs/s, pack_ms, their own byte model, a bounded CPU baseline.
   --scaling strong one fixed batch partitioned by arc count over the ranks (shard.py).
+  --dump-outputs   what the last timed step computed, as .npy files (dump_outputs()): the inputs
+                   are seeded, so two builds run with the same arguments compare output for output.
 """
 import argparse
 import json
@@ -203,32 +205,36 @@ def run_tool(eng, klu, tool, flags):
         eng.run(TOOLS[tool], **flags)
 
 
-def fetch_for(eng, klu, tool, out=None):
-    """(rows, bytes brought to the host) of the last run."""
+def fetch_arrays(eng, klu, tool, out=None):
+    """The arrays the last run of `tool` hands to a caller (klu_fetch_*)."""
     t = TOOLS[tool]
     if t == klu.FRAME_POST:
         # the rows as the reference's Posterior holds them: per-frame row offsets instead of a frame column
-        r = eng.fetch_frame_post_csr(out=out)
-    elif t == klu.SEGMENT:
-        r = eng.fetch_segment()
-    elif t == klu.POSITION:
-        r = eng.fetch_position()
-    elif t == klu.POSITION_POST:
-        r = eng.fetch_position_post()
-    elif t == klu.UTTERANCE:
-        r = eng.fetch_utterance()
-    elif t == klu.FWD_BWD:
-        r = eng.fetch_fwd_bwd()
-        return 0, sum(int(x.nbytes) for x in r)
-    elif t in (klu.PRUNE_DYN_BEAM, klu.PRUNE_ARCS):
-        r = eng.fetch_prune()
-    elif t == klu.BEST_PATH2:
-        r = eng.fetch_best_path2()
-    elif t == klu.CHAR_POSITION:
-        r = eng.fetch_char_position()
-    else:
-        raise ValueError(tool)
-    return int(r[0][-1]), sum(int(x.nbytes) for x in r)
+        return eng.fetch_frame_post_csr(out=out)
+    if t == klu.SEGMENT:
+        return eng.fetch_segment()
+    if t == klu.POSITION:
+        return eng.fetch_position()
+    if t == klu.POSITION_POST:
+        return eng.fetch_position_post()
+    if t == klu.UTTERANCE:
+        return eng.fetch_utterance()
+    if t == klu.FWD_BWD:
+        return eng.fetch_fwd_bwd()
+    if t in (klu.PRUNE_DYN_BEAM, klu.PRUNE_ARCS):
+        return eng.fetch_prune()
+    if t == klu.BEST_PATH2:
+        return eng.fetch_best_path2()
+    if t == klu.CHAR_POSITION:
+        return eng.fetch_char_position()
+    raise ValueError(tool)
+
+
+def fetch_for(eng, klu, tool, out=None):
+    """(rows, bytes brought to the host) of the last run."""
+    r = fetch_arrays(eng, klu, tool, out)
+    rows = 0 if TOOLS[tool] == klu.FWD_BWD else int(r[0][-1])
+    return rows, sum(int(x.nbytes) for x in r)
 
 
 def time_steps(eng, klu, tool, flags, steps, warmup):
@@ -239,6 +245,78 @@ def time_steps(eng, klu, tool, flags, steps, warmup):
     for _ in range(steps):
         run_tool(eng, klu, tool, flags)
     return eng.timer_stop() / steps
+
+
+DUMP_BYTES = 63 * 10**6  # under 64 MB with the .npy headers
+DUMP_LATTICES = 64
+
+
+def dump_outputs(eng, klu, tool, batch, d):
+    """Writes what the last run of `tool` hands to a caller as DIR/<name>.npy: the per-lattice arrays of
+    the whole batch, and the per-row / per-state arrays of a fixed, seeded sample of lattices (at most 64,
+    fewer where their rows would take the files past 64 MB; `sample.npy` lists them).  Floats keep their
+    dtype, integers are stored as float64 (exact).  Returns (sampled lattices, bytes written)."""
+    nlat = len(batch)
+    t = TOOLS[tool]
+    r = fetch_arrays(eng, klu, tool)
+    if t == klu.FWD_BWD:
+        al, be, tot = r
+        whole = {"total": tot}
+        parts = {"alpha": (al, batch.state_off), "beta": (be, batch.state_off)}
+    else:
+        off = r[0]
+        whole = {"rows": np.diff(off)}
+
+        def by_row(names, xs):
+            return {k: (x, off) for k, x in zip(names, xs)}
+
+        if t == klu.FRAME_POST:
+            _, nf, fo, w, lp = r
+            whole["num_frames"] = nf
+            slots = np.concatenate([[0], np.cumsum(nf.astype(np.int64) + 1)])
+            parts = {"frame_row_off": (fo, slots), "word": (w, off), "logp": (lp, off)}
+        elif t == klu.SEGMENT:
+            parts = by_row(("word", "t0", "t1", "logp"), r[1:])
+        elif t == klu.POSITION:
+            parts = by_row(("word", "pos", "t0", "t1", "logp"), r[1:])
+        elif t == klu.POSITION_POST:
+            whole["num_pos"] = r[1]
+            parts = by_row(("pos", "word", "logp"), r[2:])
+        elif t == klu.UTTERANCE:
+            parts = by_row(("word", "logp"), r[1:])
+        elif t == klu.BEST_PATH2:
+            whole["cost"], whole["num_frames"] = r[2], r[3]
+            parts = by_row(("label",), r[1:2])
+        elif t in (klu.PRUNE_DYN_BEAM, klu.PRUNE_ARCS):
+            _, ai, ns, nd, g, a, smap, fg, fa, beams = r
+            whole["beams"] = beams.reshape(nlat, 2)
+            parts = by_row(("arc", "src", "dst", "graph", "acoustic"), (ai, ns, nd, g, a))
+            per_state = zip(("state_map", "fin_graph", "fin_acoustic"), (smap, fg, fa))
+            parts.update({k: (x, batch.state_off) for k, x in per_state})
+        elif t == klu.CHAR_POSITION:
+            _, coff, chars, pos, t0, t1, lp = r
+            parts = by_row(("num_chars", "pos", "t0", "t1", "logp"), (np.diff(coff), pos, t0, t1, lp))
+            parts["chars"] = (chars, coff[off])
+        else:
+            raise ValueError(tool)
+
+    def out(x):
+        return x if x.dtype in (np.float32, np.float64) else x.astype(np.float64)
+
+    budget = DUMP_BYTES - sum(out(x).nbytes for x in whole.values()) - 8 * min(nlat, DUMP_LATTICES)
+    cost = np.zeros(nlat, np.int64)
+    for x, o in parts.values():
+        cost += np.diff(np.asarray(o, np.int64)) * out(x[:0]).itemsize
+    order = np.random.RandomState(0x5EED).permutation(nlat)[:DUMP_LATTICES]
+    sample = np.sort(order[:int(np.searchsorted(np.cumsum(cost[order]), budget, side="right"))])
+    files = {k: out(np.asarray(x)) for k, x in whole.items()}
+    files["sample"] = sample.astype(np.float64)
+    for k, (x, o) in parts.items():
+        files[k] = out(np.concatenate([x[:0]] + [x[int(o[l]):int(o[l + 1])] for l in sample]))
+    os.makedirs(d, exist_ok=True)
+    for k, x in files.items():
+        np.save(os.path.join(d, k + ".npy"), x)
+    return len(sample), sum(x.nbytes for x in files.values())
 
 
 def kernel_profile(eng, klu, tool, flags, runs=2):
@@ -495,8 +573,14 @@ def main():
     ap.add_argument("--no-tools", action="store_true", help="skip the per-tool section")
     ap.add_argument("--tools-steps", type=int, default=3)
     ap.add_argument("--tools-scale", type=float, default=1.0, help="scales the per-tool lattice counts")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0's shard) as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm counts rows and returns no arrays")
 
     if args.impl == "reference":
         rank = int(os.environ.get("RANK", "0"))
@@ -583,6 +667,10 @@ def main():
     pack_total = reduce_max(pack_total)
     entries, _ = fetch_for(eng, klu, args.tool)
     value = total_arcs / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        nsample, nbytes = dump_outputs(eng, klu, args.tool, batch, args.dump_outputs)
+        sys.stderr.write("bench: outputs of the last timed step (%d sampled lattices, %d bytes) in %s\n"
+                         % (nsample, nbytes, args.dump_outputs))
 
     # ---- per-kernel profile (CUDA events on the launching stream) ----
     prof = kernel_profile(eng, klu, args.tool, flags, 2)
