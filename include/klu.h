@@ -18,6 +18,8 @@
  *                      (+ kwsbin2/utils.h:41-303, fstext/fstext-utils2.h:278-603)
  *   KLU_POSITION_POST  latbin/lattice-to-word-position-post.cc:70-141 (SURVEY.md 8f)
  *   KLU_CHAR_SEGMENT   kwsbin2/lattice-char-index-segment.cc:93-223 (SURVEY.md 8f)
+ *                      (both char tools: the pseudo-word frontier is bounded by --nbest, see
+ *                      klu_opts.nbest)
  *   KLU_LENGTH_DIST    latbin/lattice-to-transcript-length-dist.cc:64-125 (SURVEY.md 8f)
  *   KLU_PRUNE_ARCS     latbin/lattice-prune-arcs.cc:34-84,136-165 (SURVEY.md 8f)
  *
@@ -108,7 +110,12 @@ typedef struct klu_opts {
   float min_beam;     /* --min-beam   1e-3  (prune-dyn-beam) */
   int32_t max_arcs;   /* --max-arcs   INT_MAX */
   int32_t max_states; /* --max-states INT_MAX */
-  int32_t nbest;      /* --nbest 100 (char index) */
+  int32_t nbest;      /* --nbest 100 (char index).  Also bounds the work: a pseudo-word prefix
+                       * none of whose extensions can still reach a lattice's nbest best rows is
+                       * not expanded (an exact cut: the rows and their order are those of the
+                       * uncut search).  A lattice fails with "more than 2^24 trie nodes at one
+                       * depth" only when nbest is not below its row count and its uncut frontier
+                       * is that large. */
   /* char index label groups (kwsbin2/utils.h:41-84): parallel arrays label->group
    * (epsilon->0 and whitespace->1 included by the caller), the groups that
    * increment the word count (INT_MAX = default group, 2, 3, ...), and the

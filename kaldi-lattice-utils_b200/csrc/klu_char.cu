@@ -58,6 +58,7 @@ struct CharArgs {
   const int64_t* cell_base;    // [L] first cell of each lattice
   double* A;                   // split forward scores
   double* exitw;               // [S * NG]
+  double* cont;                // [S * NG] in-group continuation mass C (k_char_cont)
 };
 
 __device__ __forceinline__ int group_of(const CharArgs& a, int label) {
@@ -264,6 +265,34 @@ __global__ void __launch_bounds__(256) k_char_exit(CharArgs a) {
   }
 }
 
+// ---- 3b. in-group continuation mass (the n-best cut, see "frontier cut" below) ------
+// C[x][g] = LogAdd(exit[x][g], sum over arcs x -> y with group g that k_char_count / k_char_expand
+// follow (same costs, same beam test) of -cost + C[y][g]): the log-sum of every way a pseudo-word
+// of group g that has reached x can still go on and end.  The backward twin of k_char_fwd: one CTA
+// per lattice, levels in descending order, a thread per (state, group) of the level.
+__global__ void __launch_bounds__(256) k_char_cont(CharArgs a) {
+  const BatchView& b = a.b;
+  const int l = blockIdx.x;
+  const int* lv = b.lvl_start + b.lvl_off[l];
+  const int nl = b.lvl_off[l + 1] - b.lvl_off[l] - 1;
+  const int NG = a.NG;
+  for (int j = nl - 1; j >= 0; --j) {
+    const int a0 = lv[j], a1 = lv[j + 1];
+    for (int t = threadIdx.x; t < (a1 - a0) * NG; t += blockDim.x) {
+      const int x = a0 + t / NG, g = t % NG;
+      double acc = a.exitw[(long long)x * NG + g];
+      for (int k = b.out_off[x]; k < b.out_off[x + 1]; ++k) {
+        const int4 r = b.out_rec[k];
+        if (group_of(a, r.w) != g || char_arc_pruned(a, l, x, r.x, r)) continue;
+        const double y = a.cont[(long long)r.x * NG + g];
+        if (y > neg_inf()) acc = log_add(acc, y - rec_cost(r, a.cp));
+      }
+      a.cont[(long long)x * NG + g] = acc;
+    }
+    __syncthreads();
+  }
+}
+
 // ---- 4. frontier determinisation ---------------------------------------------------
 struct Frontier {
   // items of the current depth: lattice l owns [ibase[l], ibase[l] + icnt[l])
@@ -299,7 +328,57 @@ struct Frontier {
   int64_t node_pool_base;   // first pool slot of the depth being created
   int64_t parent_pool_base; // first pool slot of the current depth (parents)
   int depth;
+  // n-best cut (see "frontier cut" below)
+  double* nd_ub;            // per node: subtree bound U
+  const double* tau;        // [L] cut threshold tau (log-probability); nullptr = no cut
+  int32_t* tk_cnt;          // [L] keys in the lattice's threshold segment; nullptr = no keys gathered
+  const int32_t* tk_keep;   // [L] of them carried over from the last depth
+  const int64_t* tk_wbase;  // [L] threshold segment (work buffer)
+  const int64_t* tk_tbase;  // [L] carried-over keys (top buffer)
+  unsigned long long* tk_work;
+  const unsigned long long* tk_top;
+  unsigned long long* cut_cnt;  // KLU_CHAR_DEBUG: candidates cut at this depth (else nullptr)
 };
+
+// ---- frontier cut --------------------------------------------------------------------
+// Only the nbest best rows (trie nodes) of a lattice are kept, so a prefix none of whose
+// extensions can reach them need not be expanded.  Exact bound (items (p, x, wsum) of node p of
+// group g, exit[x][g], nd_total(p) = log-sum over the items of wsum + exit, k_char_accum):
+//   1. C[x][g] (k_char_cont) is the log-sum over every in-group continuation of x, along the very
+//      arcs and costs that k_char_count / k_char_expand follow, ended by an exit.
+//   2. U(p) = log-sum over ALL items of p (exit -inf included) of wsum + C[x][g].  Every sub-path
+//      that spells p or a descendant q of p passes through exactly one item of p and goes on along
+//      such arcs, so U(p) >= nd_total(q) for every q of p's subtree.  Position keys (word count)
+//      and segment keys (frame tags) only split the sub-paths further; the bound holds for both.
+//   3. tau_l = the nbest-th largest row log-probability (nd_total - beta[start], as k_char_rowkey
+//      forms it) among the lattice's final nodes; -inf until there are nbest of them.  The nodes
+//      of a depth are final once k_char_accum has folded them; tau only rises.
+//   4. An item of a node with U(p) - beta[start] < tau_l - delta emits no candidates.  The node
+//      itself stays a row candidate; it is below tau, so it is never selected.
+//   5. Every node whose log-probability is >= the final tau survives (rounding is monotone, so
+//      U >= total gives U - beta >= total - beta).  Survivors keep their order inside a lattice
+//      (depth, then key order: removing emptied parents renumbers the rest monotonically), so the
+//      two stable row sorts and k_char_select pick the same nodes, ties at the cut included.
+//   6. delta absorbs rounding: U and the totals are f64 sums of the same terms taken in different
+//      orders.  An add or log_add rounds within 2 ulp of its result, and an error passes through a
+//      later log_add with a factor <= 1; every sum reaches a row through fewer than 2^31 such steps
+//      (the batch's work-item limit), whose operands are bounded by M = 1 + |tau| + |beta[start]|.
+//      So U and a total differ from their exact values by < 2 * 2^31 * 2^-51 * M = 2^-19 M;
+//      delta = 2^-16 M is eight times that.  delta only keeps more, so it cannot change a result.
+// With nbest at least the rows a lattice ends up with, tau stays -inf and nothing is cut.
+constexpr double kCutSlack = 1.0 / 65536.0;
+
+__device__ __forceinline__ bool below_cut(double ub_logp, double tau, double beta0) {
+  if (!(tau > neg_inf())) return false;
+  if (tau == pos_inf()) return true;  // nbest 0: no row is selected
+  return ub_logp < tau - kCutSlack * (1.0 + fabs(tau) + fabs(beta0));
+}
+
+// inverse of ~ord_f64: the log-probability of a threshold key
+__device__ __forceinline__ double key_logp(unsigned long long k) {
+  const unsigned long long u = ~k;
+  return __longlong_as_double((long long)((u & 0x8000000000000000ULL) ? (u & 0x7fffffffffffffffULL) : ~u));
+}
 
 // lattice-char-index-segment: SymbolToPathSegmentationFst (kwsbin2/utils.h:251-303) keeps
 // an output label on every arc that enters a state where the sub-path may stop (a final
@@ -367,35 +446,84 @@ __global__ void __launch_bounds__(256) k_char_emit0(CharArgs a, Frontier f) {
 }
 
 // node scores of the current depth: the first item of every node folds the node's
-// items (they are sorted by state) with their exit weights
+// items (they are sorted by state) with their exit weights, and the subtree bound U.
+// With the cut on, rows above tau go to the lattice's threshold segment, after the keys
+// carried over from the last depth (copied here from the top buffer).
 __global__ void __launch_bounds__(256) k_char_accum(CharArgs a, Frontier f) {
   const LatTile lt = lat_tile();  // CTAs that run together share lattices (L2 locality)
   const int l = lt.l;
   const int n = f.icnt[l];
   const int64_t base = f.ibase[l];
-  for (int i = lt.tile * blockDim.x + threadIdx.x; i < n; i += lt.tiles * blockDim.x) {
-    const int node = f.it_node[base + i];
-    if (i > 0 && f.it_node[base + i - 1] == node) continue;
-    const int g = f.nd_grp[node];
-    double total = neg_inf(), best = neg_inf();
-    int t0 = 0, t1 = 0;
-    for (int q = i; q < n && f.it_node[base + q] == node; ++q) {
-      const int x = f.it_state[base + q];
-      const double ex = a.exitw[(long long)x * a.NG + g];
-      if (!(ex > neg_inf())) continue;
-      total = log_add(total, f.it_wsum[base + q] + ex);
-      const double v = f.it_wmax[base + q] + ex;
-      const int q0 = f.it_t0[base + q], q1 = a.b.time[x];
-      if (v > best || (v == best && (q0 < t0 || (q0 == t0 && q1 < t1)))) {
-        best = v;
-        t0 = q0;
-        t1 = q1;
+  const int lane = threadIdx.x & 31;
+  const double beta0 = a.beta[a.b.s_off[l]];
+  const double tau = f.tk_cnt ? f.tau[l] : 0.0;
+  if (f.tk_cnt) {
+    const int keep = f.tk_keep[l];
+    const int64_t wb = f.tk_wbase[l], tb = f.tk_tbase[l];
+    for (int j = lt.tile * blockDim.x + threadIdx.x; j < keep; j += lt.tiles * blockDim.x) f.tk_work[wb + j] = f.tk_top[tb + j];
+  }
+  // warp-uniform trip count: the threshold keys are appended with one atomic per warp
+  for (int i0 = lt.tile * blockDim.x + (threadIdx.x & ~31); i0 < n; i0 += lt.tiles * blockDim.x) {
+    const int i = i0 + lane;
+    bool pass = false;
+    double logp = 0.0;
+    const int node = i < n ? f.it_node[base + i] : -1;
+    if (i < n && !(i > 0 && f.it_node[base + i - 1] == node)) {
+      const int g = f.nd_grp[node];
+      double total = neg_inf(), best = neg_inf(), ub = neg_inf();
+      int t0 = 0, t1 = 0;
+      for (int q = i; q < n && f.it_node[base + q] == node; ++q) {
+        const int x = f.it_state[base + q];
+        const double cx = a.cont[(long long)x * a.NG + g];
+        if (cx > neg_inf()) ub = log_add(ub, f.it_wsum[base + q] + cx);
+        const double ex = a.exitw[(long long)x * a.NG + g];
+        if (!(ex > neg_inf())) continue;
+        total = log_add(total, f.it_wsum[base + q] + ex);
+        const double v = f.it_wmax[base + q] + ex;
+        const int q0 = f.it_t0[base + q], q1 = a.b.time[x];
+        if (v > best || (v == best && (q0 < t0 || (q0 == t0 && q1 < t1)))) {
+          best = v;
+          t0 = q0;
+          t1 = q1;
+        }
+      }
+      f.nd_total[node] = total;
+      f.nd_best[node] = best;
+      f.nd_t0[node] = t0;
+      f.nd_t1[node] = t1;
+      f.nd_ub[node] = ub;
+      logp = total - beta0;  // as k_char_rowkey forms it
+      pass = total > neg_inf() && logp > tau;
+    }
+    if (f.tk_cnt) {
+      const unsigned int m = __ballot_sync(0xffffffffu, pass);
+      if (m) {
+        const int leader = __ffs(m) - 1;
+        int first = 0;
+        if (lane == leader) first = atomicAdd(f.tk_cnt + l, __popc(m));
+        first = __shfl_sync(0xffffffffu, first, leader);
+        if (pass) f.tk_work[f.tk_wbase[l] + first + __popc(m & ((1u << lane) - 1u))] = ~ord_f64(logp + 0.0);
       }
     }
-    f.nd_total[node] = total;
-    f.nd_best[node] = best;
-    f.nd_t0[node] = t0;
-    f.nd_t1[node] = t1;
+  }
+}
+
+// after the sort of the threshold segments (descending log-probability): the nbest best keys
+// are carried over to the top buffer, and tau becomes the nbest-th once there are nbest of them
+// (unsorted = no segment can hold nbest keys yet: all are carried over, tau stays)
+__global__ void __launch_bounds__(256) k_char_tau(Frontier f, const unsigned long long* key_b, const unsigned char* where,
+                                                  int sorted, int nbest, unsigned long long* top, int32_t* keep_out,
+                                                  double* tau) {
+  const int l = blockIdx.x;
+  const int n = f.tk_cnt[l];
+  const int keep = min(n, nbest);
+  const unsigned long long* src = (sorted && where[l] ? key_b : f.tk_work) + f.tk_wbase[l];
+  for (int j = threadIdx.x; j < keep; j += blockDim.x) top[f.tk_tbase[l] + j] = src[j];
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    if (sorted && n >= nbest) tau[l] = key_logp(src[nbest - 1]);
+    keep_out[l] = keep;
+    f.tk_cnt[l] = keep;
   }
 }
 
@@ -406,13 +534,25 @@ __global__ void __launch_bounds__(256) k_char_count(CharArgs a, Frontier f) {
   const int l = lt.l;
   const int n = f.icnt[l];
   const int64_t base = f.ibase[l];
+  const double beta0 = a.beta[b.s_off[l]];
+  const double tau = f.tau ? f.tau[l] : neg_inf();
   for (int i = lt.tile * blockDim.x + threadIdx.x; i < n; i += lt.tiles * blockDim.x) {
     const int x = f.it_state[base + i];
-    const int g = f.nd_grp[f.it_node[base + i]];
+    const int node = f.it_node[base + i];
+    const bool cut = below_cut(f.nd_ub[node] - beta0, tau, beta0);
+    if (cut && !f.cut_cnt) {
+      f.cand_cnt[base + i] = 0;
+      continue;
+    }
+    const int g = f.nd_grp[node];
     int c = 0;
     for (int k = b.out_off[x]; k < b.out_off[x + 1]; ++k) {
       const int4 r = b.out_rec[k];
       if (group_of(a, r.w) == g && !char_arc_pruned(a, l, x, r.x, r)) ++c;
+    }
+    if (cut) {  // counted for the debug line only
+      if (c) atomicAdd(f.cut_cnt, (unsigned long long)c);
+      c = 0;
     }
     f.cand_cnt[base + i] = c;
   }
@@ -824,7 +964,7 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
     gdense.push_back(kv.second);
   }
   const size_t S = (size_t)c->S, E = (size_t)std::max<int64_t>(c->E, 1);
-  enum { C_GL = 0, C_GD, C_NLO, C_NHI, C_CCNT, C_CLOC, C_CBASE, C_A, C_EXIT, C_TOT, C_MISC };
+  enum { C_GL = 0, C_GD, C_NLO, C_NHI, C_CCNT, C_CLOC, C_CBASE, C_A, C_EXIT, C_TOT, C_CONT };
   DevBuf* sc = c->d_scratch;
   KLU_TRY(sc[C_GL].reserve(4 * glabels.size()));
   KLU_TRY(sc[C_GD].reserve(4 * glabels.size()));
@@ -911,6 +1051,13 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
     k_char_exit<<<dim3(L, st_tiles), 256, 0, c->stream>>>(a);
   }
   KLU_TRY(check_launch("k_char_exit"));
+  KLU_TRY(sc[C_CONT].reserve(8 * S * (size_t)a.NG));
+  a.cont = sc[C_CONT].as<double>();
+  {
+    KLU_LAUNCH(c, "k_char_cont");
+    k_char_cont<<<L, 256, 0, c->stream>>>(a);
+  }
+  KLU_TRY(check_launch("k_char_cont"));
 
   // ---- frontier buffers (grown as needed) ----
   // The frontier, trie and row buffers live in the context (c->d_char) and are reused from run to
@@ -922,9 +1069,13 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
   DevBuf &ckey_a = buf(), &ckey_b = buf(), &cval_a = buf(), &cval_b = buf(), &c_wsum = buf(), &c_wmax = buf(),
          &c_t0 = buf(), &c_state = buf(), &c_main = buf(), &cand_cnt = buf(), &cand_loc = buf(), &where = buf();
   DevBuf &nd_parent = buf(), &nd_chr = buf(), &nd_cnt = buf(), &nd_grp = buf(), &nd_lat = buf(), &nd_t0 = buf(),
-         &nd_t1 = buf(), &nd_len = buf(), &nd_total = buf(), &nd_best = buf();
+         &nd_t1 = buf(), &nd_len = buf(), &nd_total = buf(), &nd_best = buf(), &nd_ub = buf();
   DevBuf &d_ibase = buf(), &d_icnt = buf(), &d_cbase = buf(), &d_ccnt = buf(), &d_ncnt = buf();
   DevBuf &tile_i = buf(), &tile_n = buf();
+  // n-best cut: per-lattice threshold segments (work keys + sort buffers), carried-over keys (top),
+  // [L] counts / tau, [3 (L+1)] bases (work, top of the last depth, top of this depth), debug count
+  DevBuf &tk_work = buf(), &tk_keyb = buf(), &tk_vala = buf(), &tk_valb = buf(), &tk_top = buf(), &tk_where = buf(),
+         &tk_cnt = buf(), &tk_keep = buf(), &tk_tau = buf(), &tk_bases = buf(), &d_cut = buf();
   KLU_TRY(d_ibase.reserve(8 * (size_t)(L + 1)));
   KLU_TRY(d_icnt.reserve(4 * (size_t)L));
   KLU_TRY(d_cbase.reserve(8 * (size_t)(L + 1)));
@@ -934,9 +1085,9 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
   KLU_TRY(cand_cnt.reserve(4 * E));
   KLU_TRY(cand_loc.reserve(4 * E));
   int64_t pool = 0;  // node pool slots in use
-  DevBuf* nd_all[10] = {&nd_parent, &nd_chr, &nd_cnt, &nd_grp, &nd_lat, &nd_t0, &nd_t1, &nd_len, &nd_total, &nd_best};
+  DevBuf* nd_all[11] = {&nd_parent, &nd_chr, &nd_cnt, &nd_grp, &nd_lat, &nd_t0, &nd_t1, &nd_len, &nd_total, &nd_best, &nd_ub};
   auto grow_pool = [&](int64_t need) -> int {
-    for (int i = 0; i < 10; ++i) {
+    for (int i = 0; i < 11; ++i) {
       const size_t w = i >= 8 ? 8 : 4;
       KLU_TRY(grow_keep(c, *nd_all[i], (size_t)pool * w, (size_t)need * w));
     }
@@ -947,6 +1098,87 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
   int64_t items_total = 0;            // slots of the current item arrays
   std::vector<int32_t> h_cnt(L);
   int64_t parent_pool_base = 0;
+  // n-best cut state: tau starts at -inf (+inf with nbest 0: no row is selected, nothing is
+  // expanded); a lattice's threshold keys are gathered from depth 1 on
+  const int nbest = o->nbest;
+  const bool debug = getenv("KLU_CHAR_DEBUG") != nullptr;
+  std::vector<int64_t> h_seen(L, 0);  // items folded so far per lattice (>= its final nodes)
+  std::vector<int64_t> h_tkb(3 * (size_t)(L + 1), 0);  // work | top of the last depth | top of this depth
+  KLU_TRY(tk_cnt.reserve(4 * (size_t)L));
+  KLU_TRY(tk_keep.reserve(4 * (size_t)L));
+  KLU_TRY(tk_tau.reserve(8 * (size_t)L));
+  KLU_TRY(tk_where.reserve((size_t)L));
+  KLU_TRY(tk_bases.reserve(8 * h_tkb.size()));
+  KLU_TRY(d_cut.reserve(8));
+  {
+    const std::vector<double> tau0(L, nbest > 0 ? -INFINITY : INFINITY);
+    KLU_CUDA(cudaMemcpyAsync(tk_tau.p, tau0.data(), 8 * (size_t)L, cudaMemcpyHostToDevice, c->stream));
+    KLU_CUDA(cudaMemsetAsync(tk_cnt.p, 0, 4 * (size_t)L, c->stream));
+    KLU_CUDA(cudaMemsetAsync(tk_keep.p, 0, 4 * (size_t)L, c->stream));
+    KLU_CUDA(cudaStreamSynchronize(c->stream));  // tau0 leaves scope
+  }
+  f.tau = tk_tau.as<double>();
+  f.tk_keep = tk_keep.as<int32_t>();
+  f.tk_wbase = tk_bases.as<int64_t>();
+  f.tk_tbase = tk_bases.as<int64_t>() + (L + 1);
+  unsigned long long h_cut = 0;
+  // threshold step of one depth: lay out the segments (carried-over keys + this depth's items per
+  // lattice), let k_char_accum fill them, sort, carry the nbest best over and update tau
+  auto cut_layout = [&]() -> int {
+    int64_t w = 0, t = 0;
+    for (int32_t l = 0; l <= L; ++l) h_tkb[(size_t)(L + 1) + l] = h_tkb[2 * (size_t)(L + 1) + l];  // top of the last depth
+    const int64_t t_last = h_tkb[2 * (size_t)(L + 1) - 1];
+    for (int32_t l = 0; l < L; ++l) {
+      h_tkb[l] = w;
+      w += std::min<int64_t>(nbest, h_seen[l]) + h_cnt[l];
+      h_seen[l] += h_cnt[l];
+      h_tkb[2 * (size_t)(L + 1) + l] = t;
+      t += std::min<int64_t>(nbest, h_seen[l]);
+    }
+    h_tkb[L] = w;
+    h_tkb[2 * (size_t)(L + 1) + L] = t;
+    KLU_TRY(tk_work.reserve(8 * (size_t)std::max<int64_t>(w, 1)));
+    KLU_TRY(tk_keyb.reserve(8 * (size_t)std::max<int64_t>(w, 1)));
+    KLU_TRY(tk_vala.reserve(4 * (size_t)std::max<int64_t>(w, 1)));
+    KLU_TRY(tk_valb.reserve(4 * (size_t)std::max<int64_t>(w, 1)));
+    // the top buffer keeps the last depth's keys until k_char_accum has copied them
+    KLU_TRY(grow_keep(c, tk_top, 8 * (size_t)t_last, 8 * (size_t)std::max<int64_t>(std::max(t, t_last), 1)));
+    KLU_CUDA(cudaMemcpyAsync(tk_bases.p, h_tkb.data(), 8 * h_tkb.size(), cudaMemcpyHostToDevice, c->stream));
+    f.tk_work = tk_work.as<unsigned long long>();
+    f.tk_top = tk_top.as<unsigned long long>();
+    f.tk_tbase = tk_bases.as<int64_t>() + (L + 1);
+    return 0;
+  };
+  auto cut_update = [&]() -> int {
+    bool full = false;  // some lattice may hold nbest keys: sort
+    for (int32_t l = 0; l < L; ++l) full = full || h_seen[l] >= nbest;
+    SegSortArgs ss;
+    ss.seg_base = tk_bases.as<int64_t>();
+    ss.seg_cnt = tk_cnt.as<int32_t>();
+    ss.key_a = tk_work.as<unsigned long long>();
+    ss.val_a = tk_vala.as<unsigned int>();
+    ss.key_b = tk_keyb.as<unsigned long long>();
+    ss.val_b = tk_valb.as<unsigned int>();
+    ss.where = tk_where.as<unsigned char>();
+    ss.lo_bit = 0;
+    ss.hi_bit = 64;
+    if (full) {
+      {
+        KLU_LAUNCH(c, "k_seg_radix_sort");
+        KLU_TRY(seg_sort_launch(c, ss, L, h_tkb[L]));
+      }
+      KLU_TRY(check_launch("k_seg_radix_sort(char cut)"));
+    }
+    Frontier g = f;
+    g.tk_tbase = tk_bases.as<int64_t>() + 2 * (L + 1);  // this depth's top layout
+    {
+      KLU_LAUNCH(c, "k_char_tau");
+      k_char_tau<<<L, 256, 0, c->stream>>>(g, ss.key_b, ss.where, full ? 1 : 0, nbest, tk_top.as<unsigned long long>(),
+                                           tk_keep.as<int32_t>(), tk_tau.as<double>());
+    }
+    KLU_TRY(check_launch("k_char_tau"));
+    return 0;
+  };
   for (int depth = 0; depth < 100000; ++depth) {
     // ---- candidates: count, scan ----
     if (depth == 0) {
@@ -964,11 +1196,20 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
       KLU_TRY(cand_loc.reserve(4 * (size_t)std::max<int64_t>(items_total, 1)));
       f.cand_cnt = cand_cnt.as<int32_t>();
       f.cand_loc = cand_loc.as<int32_t>();
+      if (nbest > 0) {
+        KLU_TRY(cut_layout());
+        f.tk_cnt = tk_cnt.as<int32_t>();
+      }
       {
         KLU_LAUNCH(c, "k_char_accum");
         k_char_accum<<<dim3(L, 64), 256, 0, c->stream>>>(a, f);
       }
       KLU_TRY(check_launch("k_char_accum"));
+      if (nbest > 0) KLU_TRY(cut_update());
+      if (debug) {
+        KLU_CUDA(cudaMemsetAsync(d_cut.p, 0, 8, c->stream));
+        f.cut_cnt = d_cut.as<unsigned long long>();
+      }
       {
         KLU_LAUNCH(c, "k_char_count");
         k_char_count<<<dim3(L, 64), 256, 0, c->stream>>>(a, f);
@@ -978,11 +1219,15 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
       KLU_TRY(scan(rg, f.cand_cnt, cand_loc.as<int32_t>(), d_cbase.as<int64_t>()));
     }
     const int64_t ncand = h_base[L];
-    if (getenv("KLU_CHAR_DEBUG")) {
+    if (debug) {
       long long mx = 0;
       for (int32_t l = 0; l < L; ++l) mx = std::max(mx, h_tot[l]);
-      fprintf(stderr, "[klu char] depth %d: %lld candidates (largest lattice %lld), pool %lld, items %lld\n", depth,
-              (long long)ncand, mx, (long long)pool, (long long)items_total);
+      if (depth > 0) {
+        KLU_CUDA(cudaMemcpyAsync(&h_cut, d_cut.p, 8, cudaMemcpyDeviceToHost, c->stream));
+        KLU_CUDA(cudaStreamSynchronize(c->stream));
+      }
+      fprintf(stderr, "[klu char] depth %d: %lld candidates (largest lattice %lld), %llu cut, pool %lld, items %lld\n",
+              depth, (long long)ncand, mx, depth > 0 ? h_cut : 0ULL, (long long)pool, (long long)items_total);
     }
     if (ncand == 0) break;
     for (int32_t l = 0; l < L; ++l) {
@@ -1025,6 +1270,7 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
     f.nd_len = nd_len.as<int32_t>();
     f.nd_total = nd_total.as<double>();
     f.nd_best = nd_best.as<double>();
+    f.nd_ub = nd_ub.as<double>();
     f.cbase = d_cbase.as<int64_t>();
     f.ccnt = d_ccnt.as<int32_t>();
     f.ckey = ckey_a.as<unsigned long long>();

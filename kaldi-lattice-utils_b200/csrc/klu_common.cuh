@@ -172,7 +172,7 @@ struct klu_ctx {
   klu::DevBuf d_scratch[12];           // tool scratch (keys, indices, values ...)
   klu::DevBuf d_res[8];                // dense results of the last run
   klu::DevBuf d_flush;
-  klu::DevBuf d_char[64];              // frontier / trie / row buffers of the character tools (klu_char.cu)
+  klu::DevBuf d_char[80];              // frontier / trie / row buffers of the character tools (klu_char.cu)
 
   // ---- last run ----
   int last_tool = -1;
