@@ -162,6 +162,7 @@ __device__ void log_sweep_tiles(const SweepArgs& a, int first, int lane, double2
     }
   if (!done && (FWD ? j >= nl : j < 0)) done = true;
   int a0 = 0, a1 = 0, s0 = 0;
+  int wide = 0x7fffffff;  // backward: first state of the nearest level above the current one wider than kRing
   if (!done) {
     s0 = a0 = lv[j];
     a1 = lv[j + 1];
@@ -187,9 +188,13 @@ __device__ void log_sweep_tiles(const SweepArgs& a, int first, int lane, double2
     // Passes over the lane's own arcs, each a batch of independent memory operations:
     // (1) the 16-byte records, global -> shared, asynchronously; (2) cost from the record
     // and the other end's score -- from the tile's shared-memory ring of recent scores
-    // when it is still there (a level [a0, a1) overwrites the ring slots of the states
-    // kRing below a0.. / above ..a1, everything nearer is intact), else gathered
-    // asynchronously into the slot -- and the exp term; (3) the exp terms of the gathered ones.
+    // when it is still there, else gathered asynchronously into the slot -- and the exp
+    // term; (3) the exp terms of the gathered ones.
+    // Ring slot t & (kRing - 1) still holds state t while no state t +- m kRing was written
+    // after it.  Forward, states are written in ascending order, so every t >= a1 - kRing
+    // is intact.  Backward, levels go down but the states of a level go up: t < a0 + kRing
+    // keeps the current level's writes off t's slot, and t < wide keeps t out of levels
+    // wider than kRing, where t + kRing of t's own level was written after t.
     for (int i = sl; i < nb; i += G) cp_async16(xbuf + i, rec + base + i);
     cp_async_wait_all();
     unsigned int pending = 0;
@@ -200,7 +205,7 @@ __device__ void log_sweep_tiles(const SweepArgs& a, int first, int lane, double2
         double cost = rec_cost(r, a.cp);
         if (BEAM && sweep_arc_pruned<FWD, BEAM>(a, l, base + i, r)) cost = pos_inf();
         const int t = r.x;
-        if (FWD ? (t >= a1 - kRing) : (t < a0 + kRing)) {
+        if (FWD ? (t >= a1 - kRing) : (t < min(a0 + kRing, wide))) {
           xbuf[i].x = fast_exp(ring[t & (kRing - 1)] - cost - ref);
         } else {
           xbuf[i].x = cost;
@@ -277,6 +282,7 @@ __device__ void log_sweep_tiles(const SweepArgs& a, int first, int lane, double2
     if (!done) {
       s0 += c > 0 ? c : 1;
       if (s0 >= a1) {
+        if (!FWD && a1 - a0 > kRing) wide = a0;
         j += FWD ? 1 : -1;
         if (FWD ? j >= nl : j < 0) {
           done = true;
@@ -385,6 +391,7 @@ __device__ void log_sweep_tiles2(const SweepArgs& a, int first, int lane, double
     }
   if (!done && (FWD ? j >= nl : j < 0)) done = true;
   int a0 = 0, a1 = 0, s0 = 0;
+  int wide = 0x7fffffff;  // backward: first state of the nearest level above wider than kRing (see log_sweep_tiles)
   if (!done) {
     s0 = a0 = lv[j];
     a1 = lv[j + 1];
@@ -420,10 +427,11 @@ __device__ void log_sweep_tiles2(const SweepArgs& a, int first, int lane, double
   while (!__all_sync(0xffffffffu, done)) {
     // ---- where the NEXT batch starts, its extent, its copy
     bool n_done = done;
-    int n_j = j, n_a0 = a0, n_a1 = a1, n_s0 = s0;
+    int n_j = j, n_a0 = a0, n_a1 = a1, n_s0 = s0, n_wide = wide;
     if (!done) {
       n_s0 = s0 + (c > 0 ? c : 1);
       if (n_s0 >= a1) {
+        if (!FWD && a1 - a0 > kRing) n_wide = a0;
         n_j = j + (FWD ? 1 : -1);
         if (FWD ? n_j >= nl : n_j < 0) {
           n_done = true;
@@ -457,7 +465,7 @@ __device__ void log_sweep_tiles2(const SweepArgs& a, int first, int lane, double
         double cost = rec_cost(r, a.cp);
         if (BEAM && sweep_arc_pruned<FWD, BEAM>(a, l, base + i, r)) cost = pos_inf();
         const int t = r.x;
-        if (FWD ? (t >= a1 - kRing) : (t < a0 + kRing)) {
+        if (FWD ? (t >= a1 - kRing) : (t < min(a0 + kRing, wide))) {
           xbuf[i].x = fast_exp(ring[t & (kRing - 1)] - cost - ref);
         } else {
           xbuf[i].x = cost;
@@ -534,6 +542,7 @@ __device__ void log_sweep_tiles2(const SweepArgs& a, int first, int lane, double
     a0 = n_a0;
     a1 = n_a1;
     s0 = n_s0;
+    wide = n_wide;
     o_lo = n_lo;
     o_hi = n_hi;
     base = n_base;
