@@ -136,12 +136,7 @@ __global__ void __launch_bounds__(kBpThreads) k_bp_viterbi(BpArgs a) {
         __syncthreads();
         const long long c0 = ss_cell[0], c1 = ss_cell[take];
         for (long long cell = c0 + tid; cell < c1; cell += kBpThreads) {
-          int lo = 0, hi = take - 1;  // last k with ss_cell[k] <= cell
-          while (lo < hi) {
-            const int mid = (lo + hi + 1) >> 1;
-            if (ss_cell[mid] <= cell) lo = mid;
-            else hi = mid - 1;
-          }
+          const int lo = last_le(ss_cell, 0, take - 1, cell);  // last k with ss_cell[k] <= cell
           const int len = ss_lo[lo] + (int)(cell - ss_cell[lo]);
           Cand best;
           best.v = inf;
@@ -320,33 +315,6 @@ __global__ void __launch_bounds__(128) k_bp_trace(BpArgs a) {
   a.lab_cnt[l] = n;
 }
 
-__global__ void __launch_bounds__(1024) k_bp_scan(const int32_t* cnt, int L, int64_t* off) {
-  __shared__ long long warp_sum[32];
-  __shared__ long long carry_s;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) carry_s = 0;
-  __syncthreads();
-  for (int tile = 0; tile < L; tile += 1024) {
-    const int i = tile + tid;
-    const long long c = i < L ? cnt[i] : 0;
-    long long x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const long long y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    long long add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (i < L) off[i] = add + x - c;
-    __syncthreads();
-    if (tid == 1023) carry_s = add + x;
-    __syncthreads();
-  }
-  if (tid == 0) off[L] = carry_s;
-}
-
 __global__ void __launch_bounds__(128) k_bp_compact(const int64_t* lab_off, const int32_t* labels, const int32_t* cnt,
                                                     const int64_t* res_off, int32_t* dense, int L) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
@@ -433,11 +401,7 @@ int best_path2_decode(klu_ctx* c, const CostParams& cp, const BestPathChunk& ch)
   if (ch.l1 == L) {  // last chunk: dense label table
     KLU_TRY(c->d_res[5].reserve(8 * (size_t)(L + 1)));
     KLU_TRY(c->d_res[4].reserve(4 * (size_t)std::max<int64_t>(lab_off[L], 1)));
-    {
-      KLU_LAUNCH(c, "k_scan_counts");
-      k_bp_scan<<<1, 1024, 0, c->stream>>>(a.lab_cnt, L, c->d_res[5].as<int64_t>());
-    }
-    KLU_TRY(check_launch("k_bp_scan"));
+    KLU_TRY(scan_counts(c, a.lab_cnt, 0, L, c->d_res[5].as<int64_t>(), "k_scan_counts"));
     {
       KLU_LAUNCH(c, "k_bp_compact");
       k_bp_compact<<<(L * 32 + 127) / 128, 128, 0, c->stream>>>(a.lab_off, a.labels, a.lab_cnt,

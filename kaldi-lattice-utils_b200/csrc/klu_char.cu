@@ -111,7 +111,7 @@ __global__ void __launch_bounds__(256) k_char_scan(SegRange rg, const int32_t* c
   int64_t beg;
   int n;
   seg_range(rg, l, &beg, &n);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   if (tid == 0) carry_s = 0;
   __syncthreads();
   for (int tile = 0; tile < n; tile += 1024) {  // four consecutive elements per thread
@@ -120,25 +120,12 @@ __global__ void __launch_bounds__(256) k_char_scan(SegRange rg, const int32_t* c
 #pragma unroll
     for (int q = 0; q < 4; ++q) cc[q] = i0 + q < n ? cnt[beg + i0 + q] : 0;
     const long long c = (long long)cc[0] + cc[1] + cc[2] + cc[3];
-    long long x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const long long y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    long long add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    long long run = add + x - c;
+    long long run = cta_exclusive_scan<long long, 256>(c, warp_sum, carry_s);
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
       if (i0 + q < n) out_loc[beg + i0 + q] = (int32_t)run;
       run += cc[q];
     }
-    __syncthreads();
-    if (tid == 255) carry_s = add + x;
-    __syncthreads();
   }
   if (tid == 0) tot[l] = carry_s;
 }
@@ -208,13 +195,7 @@ __global__ void __launch_bounds__(256) k_char_fwd(CharArgs a) {
     const int q0 = a.cell_loc[a0];
     const int q1 = a1 < s1 ? a.cell_loc[a1] : a.cell_loc[a1 - 1] + a.cell_cnt[a1 - 1];
     for (int q = q0 + lane; q < q1; q += nth) {
-      int lo = a0, hi = a1 - 1;  // last state of the level with cell_loc <= q
-      while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (a.cell_loc[mid] <= q) lo = mid;
-        else hi = mid - 1;
-      }
-      const int s = lo;
+      const int s = last_le(a.cell_loc, a0, a1 - 1, q);  // last state of the level with cell_loc <= q
       const int rel = q - a.cell_loc[s];
       const int n = a.nlo[s] + rel / NG, g = rel % NG;
       const int inc = (a.inc_mask >> g) & 1u;

@@ -253,6 +253,13 @@ int pick_group(double avg_deg);  // lanes cooperating on one state, from the mea
 
 int upload_filter(klu_ctx* c, const klu_opts* o, int* mode_out, int* n_out);
 
+// klu_core.cu: per-lattice counts -> offsets by one CTA (launched and counted as `label`):
+// off[l] = off[l0] + cnt[l0] + ... + cnt[l - 1] for l in (l0, l1].  With l0 > 0, off[l0] must hold
+// the total of the lattices before l0 (a chunked run); with l0 == 0 the scan starts from 0 and
+// does not read off[0].  off may be cnt itself (the packer's totals, scanned in place).
+int scan_counts(klu_ctx* c, const int32_t* cnt, int l0, int l1, int64_t* off, const char* label);
+int scan_counts(klu_ctx* c, const long long* cnt, int l0, int l1, long long* off, const char* label);
+
 }  // namespace klu
 
 // ---------------------------------------------------------------------------
@@ -442,6 +449,41 @@ __device__ __forceinline__ bool elect_max_lane(double local_m, double m, int lan
   const unsigned int gmask = (G == 32 ? 0xffffffffu : ((1u << G) - 1u)) << ((lane / G) * G);
   const unsigned int cand = bal & gmask;
   return cand != 0 && lane == __ffs(cand) - 1;
+}
+
+// Last k in [lo, hi] with a[k] <= v, for a[] ascending over [lo, hi] (lo when none is).
+template <typename T, typename V>
+__device__ __forceinline__ int last_le(const T* a, int lo, int hi, V v) {
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (a[mid] <= v) lo = mid;
+    else hi = mid - 1;
+  }
+  return lo;
+}
+
+// Exclusive prefix sum over the NT threads of a CTA, one tile of a longer scan: returns carry + the
+// sum of x over the threads before this one, and adds the tile's sum to carry.  Every thread of the
+// CTA calls it (it holds three barriers); warp_sum and carry are __shared__, carry set before a
+// barrier.  The shuffles add in T, the carry in C.
+template <typename T, int NT, typename C = T>
+__device__ __forceinline__ C cta_exclusive_scan(T x, T (&warp_sum)[NT / 32], C& carry) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  T incl = x;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const T y = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += y;
+  }
+  if (lane == 31) warp_sum[warp] = incl;
+  __syncthreads();
+  C add = carry;
+#pragma unroll 4  // left to itself the compiler takes 16 values per trip in vector loads (+9 registers)
+  for (int w = 0; w < warp; ++w) add += warp_sum[w];
+  __syncthreads();
+  if (threadIdx.x == NT - 1) carry = add + incl;
+  __syncthreads();
+  return add + incl - x;
 }
 
 __device__ __forceinline__ int4 ld_stream(const int4* p) {

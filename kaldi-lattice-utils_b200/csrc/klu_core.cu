@@ -22,7 +22,38 @@ void stage_launch(klu_ctx* c, void* dst, const void* src, size_t bytes) {
   const int grid = (int)std::max<size_t>(1, std::min<size_t>((n + 255) / 256, 64));
   k_stage_words<<<grid, 256, 0, c->stream>>>(static_cast<uint32_t*>(dst), static_cast<const uint32_t*>(src), n);
 }
+
+// one CTA: L is small next to the arcs
+template <typename C, typename O>
+__global__ void __launch_bounds__(1024) k_scan_counts(const C* cnt, int l0, int l1, O* off) {
+  __shared__ long long warp_sum[32];
+  __shared__ long long carry;
+  if (threadIdx.x == 0) carry = l0 > 0 ? off[l0] : 0;
+  __syncthreads();
+  for (int tile = l0; tile < l1; tile += 1024) {
+    const int i = tile + threadIdx.x;
+    const long long x = cta_exclusive_scan<long long, 1024>(i < l1 ? (long long)cnt[i] : 0, warp_sum, carry);
+    if (i < l1) off[i] = x;
+  }
+  if (threadIdx.x == 0) off[l1] = carry;
+}
+
+template <typename C, typename O>
+int scan_counts_t(klu_ctx* c, const C* cnt, int l0, int l1, O* off, const char* label) {
+  {
+    KLU_LAUNCH(c, label);
+    k_scan_counts<<<1, 1024, 0, c->stream>>>(cnt, l0, l1, off);
+  }
+  return check_launch(label);
+}
 }  // namespace
+
+int scan_counts(klu_ctx* c, const int32_t* cnt, int l0, int l1, int64_t* off, const char* label) {
+  return scan_counts_t(c, cnt, l0, l1, off, label);
+}
+int scan_counts(klu_ctx* c, const long long* cnt, int l0, int l1, long long* off, const char* label) {
+  return scan_counts_t(c, cnt, l0, l1, off, label);
+}
 
 int stage_begin(klu_ctx* c, size_t L) {
   KLU_CUDA(cudaStreamSynchronize(c->stream));  // nothing in flight reads the area any more

@@ -7,22 +7,22 @@
 //
 // Which (frame, word) groups exist, which arcs feed each of them and how many rows
 // every frame emits depends only on labels and state times, not on the weights.
-// So klu_load() builds that structure ONCE per batch (build_frame_groups): the
-// arc x frame instances of a lattice sorted by (frame, word, arc), a head bit on
-// the first instance of every group, and the dense output offset of every frame.
-// A run is then three kernels:
-//   k_arc_post     p[e] = exp(fw[u] + bw[v] - cost - total): the arc's posterior,
-//                  once per arc (f64; exp(-700) ~ 1e-304 is the underflow horizon);
-//   k_group_post   one THREAD per (frame, word) group: adds the posteriors of the
-//                  group's instances in arc order (4-byte ids streamed, 8-byte
-//                  gathers of p that hit L1/L2 because neighbouring frames share
-//                  arcs) and writes (float)log(sum) to the group's pre-order row;
-//   k_frame_order  one warp per run of frames: orders the frame's rows in shared
-//                  memory (bitonic, key = ~ordered float bits << 32 | word) and
-//                  writes (frame, word, logp) to the dense table in place.
+// So klu_load() builds that structure ONCE per batch (build_frame_groups): the arcs
+// numbered by start time, the arc x frame instances of a lattice sorted by (frame,
+// word, arc), a head bit on the first instance of every group, and the dense output
+// offset of every frame.  A run is then the log sweeps and two kernels:
+//   k_frame_groups  one CTA per run of kFramesPerItem frames: the posterior
+//                   exp(fw[u] + bw[v] - cost - total) of every arc of the run's
+//                   window into shared memory (f64; exp(-700) ~ 1e-304 is the
+//                   underflow horizon), then one THREAD per (frame, word) group adds
+//                   the posteriors of the group's instances in arc order and writes
+//                   (float)log(sum) to the group's pre-order row;
+//   k_frame_order   one warp per run of frames: orders the frame's rows in shared
+//                   memory (bitonic, key = ~ordered float bits << 32 | word) and
+//                   writes (word, logp) to the dense table in place.
 // A group whose sum underflows (or is empty) is redone exactly in the log domain
-// from alpha/beta; frames with more groups than the shared-memory order buffer
-// holds are ordered in global memory (slow, same results).
+// from alpha/beta (exact_group_logp); frames with more groups than the shared-memory
+// order buffer holds are ordered in global memory (slow, same results).
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -48,20 +48,18 @@ struct FrameArgs {
   const double* alpha;
   const double* beta;
   const double* total;
-  double* parc;              // [E] per out-order arc: posterior exp(v - total)
   const int32_t* item_base;  // [L+1] first work item of each lattice
   int num_items;
   const int64_t* gloc;       // per frame slot: lattice-local first output row (T+1 per lattice)
   const int64_t* res_off;    // [L+1] first output row of each lattice
   const int32_t* gwords;     // word of every (frame, word) group, in pre-order row order (static)
   const uint32_t* gstart;    // [rows + 1] first instance of every group (static)
-  int64_t rows;
   const int4* tarc;          // [E] arcs in START-TIME order: {src, dst, graph bits, acoustic bits} (static)
   const int32_t* tlabel;     // [E] their labels; frame_arc holds indices into this order
   const int32_t* run_lo;     // per work item (run of frames): smallest / largest time-order arc index among
   const int32_t* run_hi;     // its instances (static); the arcs in between are the run's "window"
   int win_cap;               // window entries that fit the dynamic shared memory
-  int32_t *o_frame, *o_word;
+  int32_t* o_word;
   float* o_logp;
 };
 
@@ -75,15 +73,6 @@ __device__ __forceinline__ double arc_value(const FrameArgs& a, int j) {  // j: 
   const int4 t = __ldg(a.tarc + j);
   const int4 r = make_int4(t.y, t.z, t.w, __ldg(a.tlabel + j));
   return __dadd_rn(__dadd_rn(a.alpha[t.x], a.beta[t.y]), -rec_cost(r, a.cp));
-}
-
-// grid (L, tiles): the posterior of every word arc, once (cross-check path KLU_FRAME_UNFUSED)
-__global__ void __launch_bounds__(256) k_arc_post(FrameArgs a) {
-  const int l = blockIdx.x;
-  const int e0 = a.b.e_off[l], e1 = a.b.e_off[l + 1];
-  const double total = a.total[l];
-  for (int j = e0 + blockIdx.y * blockDim.x + threadIdx.x; j < e1; j += gridDim.y * blockDim.x)
-    a.parc[j] = __ldg(a.tlabel + j) != 0 ? fast_exp(arc_value(a, j) - total) : 0.0;
 }
 
 // Exact log-posterior of the group that ENDS at instance `iend` of a frame's list
@@ -180,64 +169,19 @@ __device__ void warp_sort_rows_global(float* logp, int32_t* word, int n, int lan
 }
 
 
-// one thread per (frame, word) group
-__global__ void __launch_bounds__(256) k_group_post(const __grid_constant__ FrameArgs a) {
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  const int lane = threadIdx.x & 31;
-  // the loop condition is warp-uniform: lanes past the last row idle inside the body
-  for (int64_t gw = (int64_t)blockIdx.x * blockDim.x + (threadIdx.x & ~31); gw < a.rows; gw += stride) {
-    const int64_t g = gw + lane;
-    const bool live = g < a.rows;
-    const uint32_t i0 = live ? __ldg(a.gstart + g) : 0u, i1 = live ? __ldg(a.gstart + g + 1) : 0u;
-    double sum = 0.0;
-    // four instances per trip (most groups have <= 4): the id loads, then the
-    // posterior gathers, go out together; the adds stay in arc order
-    for (uint32_t i = i0; i < i1; i += 4) {
-      unsigned int e[4];
-      double p[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) e[u] = i + u < i1 ? (unsigned int)__ldg(a.b.frame_arc + i + u) & 0x7fffffffu : 0u;
-#pragma unroll
-      for (int u = 0; u < 4; ++u) p[u] = i + u < i1 ? __ldg(a.parc + e[u]) : 0.0;
-#pragma unroll
-      for (int u = 0; u < 4; ++u) sum += p[u];
-    }
-    double lp = 0.0;
-    if (!live) {
-    } else if (sum >= 1e-280) {
-      lp = fast_log(sum);
-    } else {
-      int lo = 0, hi = a.b.L - 1;  // lattice of this row: last l with res_off[l] <= g
-      while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (a.res_off[mid] <= g) lo = mid;
-        else hi = mid - 1;
-      }
-      lp = exact_group_logp(a, a.b.frame_arc, i1 - 1, a.total[lo]);
-    }
-    if (live) a.o_logp[g] = (float)lp + 0.0f;  // -0.0 and +0.0 compare equal in the reference's sort
-  }
-}
-
 // Fused arc posteriors + group sums for one run of kFramesPerItem frames per CTA.
 // With the arcs numbered by start time (a copy made at pack time), the word arcs alive
 // in a run of frames are a contiguous index range -- the run's window.  Phase 1 computes the posterior of
 // every arc of the window into shared memory (coalesced record reads, one exp per arc;
 // windows of neighbouring runs overlap by the arcs that span the boundary, ~1/8 extra);
-// phase 2 is k_group_post with its gathers served from shared memory.  No per-arc
-// posterior array in HBM, no dependent global gathers.  Runs whose window does not fit
+// phase 2 adds each (frame, word) group's posteriors, one thread per group, from shared
+// memory.  No per-arc posterior array in HBM, no dependent global gathers.  Runs whose window does not fit
 // (very long arcs) take the posteriors from alpha/beta directly, instance by instance.
 __global__ void __launch_bounds__(128) k_frame_groups(const __grid_constant__ FrameArgs a) {
   extern __shared__ double s_post[];
   const BatchView& b = a.b;
   const int item = blockIdx.x;
-  int lo = 0, hi = b.L - 1;  // lattice of this item: last l with item_base[l] <= item
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (a.item_base[mid] <= item) lo = mid;
-    else hi = mid - 1;
-  }
-  const int l = lo;
+  const int l = last_le(a.item_base, 0, b.L - 1, item);  // lattice of this item
   const int T = b.fr_base[l + 1] - b.fr_base[l] - 1;
   const int k0 = (item - a.item_base[l]) * kFramesPerItem;
   const int k1 = min(T, k0 + kFramesPerItem);
@@ -472,14 +416,7 @@ __global__ void __launch_bounds__(kFrameWarps * 32, 8) k_frame_order(const __gri
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const BatchView& b = a.b;
   for (int item = blockIdx.x * kFrameWarps + warp; item < a.num_items; item += gridDim.x * kFrameWarps) {
-    // lattice of this item: last l with item_base[l] <= item
-    int lo = 0, hi = b.L - 1;
-    while (lo < hi) {
-      const int mid = (lo + hi + 1) >> 1;
-      if (a.item_base[mid] <= item) lo = mid;
-      else hi = mid - 1;
-    }
-    const int l = lo;
+    const int l = last_le(a.item_base, 0, b.L - 1, item);  // lattice of this item
     const int T = b.fr_base[l + 1] - b.fr_base[l] - 1;
     const int k0 = (item - a.item_base[l]) * kFramesPerItem;
     const int k1 = min(T, k0 + kFramesPerItem);
@@ -590,24 +527,14 @@ __global__ void __launch_bounds__(256) k_fg_emit(GroupArgs a) {
   const int e0 = b.e_off[l], e1 = b.e_off[l + 1];
   const int T = b.fr_base[l + 1] - b.fr_base[l] - 1;
   const int64_t base = a.inst_base[l];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   if (tid == 0) carry_s = 0;
   __syncthreads();
   for (int tile = e0; tile < e1; tile += 256) {
     const int e = tile + tid;
     int first = 0;
     const int cnt = e < e1 ? arc_frames(b, e, T, &first) : 0;
-    int x = cnt;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    int add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    const int off = add + x - cnt;
+    const int off = cta_exclusive_scan<int, 256>(cnt, warp_sum, carry_s);
     if (cnt > 0) {
       const unsigned long long word = (unsigned long long)(unsigned int)b.out_rec[e].w;
       for (int q = 0; q < cnt; ++q) {
@@ -617,9 +544,6 @@ __global__ void __launch_bounds__(256) k_fg_emit(GroupArgs a) {
         a.val[base + off + q] = (unsigned int)a.rank_of[e];
       }
     }
-    __syncthreads();
-    if (tid == 255) carry_s = add + x;
-    __syncthreads();
   }
 }
 
@@ -631,13 +555,7 @@ __global__ void __launch_bounds__(256) k_fg_heads(GroupArgs a) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const BatchView& b = a.b;
   for (int item = blockIdx.x * 8 + warp; item < a.num_items; item += gridDim.x * 8) {
-    int lo = 0, hi = b.L - 1;
-    while (lo < hi) {
-      const int mid = (lo + hi + 1) >> 1;
-      if (a.item_base[mid] <= item) lo = mid;
-      else hi = mid - 1;
-    }
-    const int l = lo;
+    const int l = last_le(a.item_base, 0, b.L - 1, item);
     const int T = b.fr_base[l + 1] - b.fr_base[l] - 1;
     const int k0 = (item - a.item_base[l]) * kFramesPerItem;
     const int k1 = min(T, k0 + kFramesPerItem);
@@ -698,58 +616,19 @@ __global__ void __launch_bounds__(256) k_fg_scan(GroupArgs a) {
   __shared__ long long carry_s;
   const int l = blockIdx.x;
   const int f0 = a.b.fr_base[l], T = a.b.fr_base[l + 1] - f0 - 1;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   if (tid == 0) carry_s = 0;
   __syncthreads();
   for (int tile = 0; tile < T; tile += 256) {
     const int k = tile + tid;
     const int c = k < T ? a.frame_cnt[f0 + k] : 0;
-    int x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    long long add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (k < T) a.gloc[f0 + k] = add + x - c;
-    __syncthreads();
-    if (tid == 255) carry_s = add + x;
-    __syncthreads();
+    const long long pre = cta_exclusive_scan<int, 256, long long>(c, warp_sum, carry_s);
+    if (k < T) a.gloc[f0 + k] = pre;
   }
   if (tid == 0) {
     a.gloc[f0 + T] = carry_s;
     a.lat_cnt[l] = (int32_t)carry_s;
   }
-}
-
-__global__ void __launch_bounds__(1024) k_fg_latscan(const int32_t* cnt, int L, int64_t* off) {
-  __shared__ long long warp_sum[32];
-  __shared__ long long carry_s;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) carry_s = 0;
-  __syncthreads();
-  for (int tile = 0; tile < L; tile += 1024) {
-    const int i = tile + tid;
-    const long long c = i < L ? cnt[i] : 0;
-    long long x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const long long y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    long long add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (i < L) off[i] = add + x - c;
-    __syncthreads();
-    if (tid == 1023) carry_s = add + x;
-    __syncthreads();
-  }
-  if (tid == 0) off[L] = carry_s;
 }
 
 int bits_for(int64_t maxv) {
@@ -807,7 +686,6 @@ int build_frame_groups(klu_ctx* c) {
   // repeated loads do not go through cudaMalloc / cudaFree again)
   DevBuf &key_a = c->d_scratch[6], &key_b = c->d_scratch[7], &val_a = c->d_scratch[8], &val_b = c->d_scratch[9],
          &misc = c->d_scratch[10];
-  auto release_all = [&]() {};
   int rc = 0;
   do {
     if ((rc = key_a.reserve(8 * (size_t)N)) || (rc = key_b.reserve(8 * (size_t)N)) ||
@@ -956,11 +834,7 @@ int build_frame_groups(klu_ctx* c) {
       k_fg_scan<<<L, 256, 0, c->stream>>>(a);
     }
     if ((rc = check_launch("k_fg_scan"))) break;
-    {
-      KLU_LAUNCH(c, "k_fg_latscan");
-      k_fg_latscan<<<1, 1024, 0, c->stream>>>(d_lat_cnt, L, c->d_fr_res_off.as<int64_t>());
-    }
-    if ((rc = check_launch("k_fg_latscan"))) break;
+    if ((rc = scan_counts(c, d_lat_cnt, 0, L, c->d_fr_res_off.as<int64_t>(), "k_fg_latscan"))) break;
     if ((rc = small_d2h(c, &c->fr_max_window, a.max_window, 4))) break;
     if ((rc = small_d2h(c, c->h_frame_res_off.data(), c->d_fr_res_off.p, 8 * (size_t)(L + 1)))) break;
     if ((rc = small_sync(c))) break;
@@ -981,7 +855,6 @@ int build_frame_groups(klu_ctx* c) {
     if ((rc = check_launch("k_fg_words"))) break;
   } while (0);
   cudaStreamSynchronize(c->stream);
-  release_all();
   return rc;
 }
 
@@ -1001,7 +874,6 @@ int run_frame_post(klu_ctx* c, const klu_opts* o) {
   c->last_entries = L ? c->h_res_off[L] : 0;
   if (L == 0) return 0;
   const int64_t N = std::max<int64_t>(c->last_entries, 1);
-  if (getenv("KLU_FRAME_UNFUSED")) KLU_TRY(c->d_scratch[0].reserve(8 * (size_t)std::max<int64_t>(c->E, 1)));
   KLU_TRY(c->d_res[5].reserve(8 * (size_t)(L + 1)));
   KLU_TRY(c->d_res[1].reserve(4 * (size_t)N));
   KLU_TRY(c->d_res[4].reserve(4 * (size_t)N));
@@ -1013,37 +885,19 @@ int run_frame_post(klu_ctx* c, const klu_opts* o) {
   a.alpha = c->d_alpha.as<double>();
   a.beta = c->d_beta.as<double>();
   a.total = c->d_total.as<double>();
-  a.parc = c->d_scratch[0].as<double>();
   a.item_base = c->d_fr_item.as<int32_t>();
   a.num_items = c->fr_items;
   a.gloc = c->d_fr_gloc.as<int64_t>();
   a.res_off = c->d_fr_res_off.as<int64_t>();
   a.gwords = c->d_fr_gword.as<int32_t>();
   a.gstart = c->d_fr_gstart.as<uint32_t>();
-  a.rows = c->last_entries;
-  a.o_frame = nullptr;  // the frame column is static per batch (d_fr_gframe)
   a.o_word = c->d_res[1].as<int32_t>();
   a.o_logp = c->d_res[4].as<float>();
   a.run_lo = c->d_fr_run_lo.as<int32_t>();
   a.run_hi = c->d_fr_run_hi.as<int32_t>();
   a.tarc = c->d_fr_tarc.as<int4>();
   a.tlabel = c->d_fr_tlabel.as<int32_t>();
-  static const bool unfused = getenv("KLU_FRAME_UNFUSED") != nullptr;  // cross-check path: posteriors through HBM
-  if (unfused) {
-    {
-      int64_t max_arcs = 0;
-      for (int32_t l = 0; l < L; ++l) max_arcs = std::max(max_arcs, c->h_e_off[l + 1] - c->h_e_off[l]);
-      const int tiles = (int)std::max<int64_t>(1, std::min<int64_t>((max_arcs + 255) / 256, 64));
-      KLU_LAUNCH(c, "k_arc_post");
-      k_arc_post<<<dim3(L, tiles), 256, 0, c->stream>>>(a);
-    }
-    KLU_TRY(check_launch("k_arc_post"));
-    {
-      KLU_LAUNCH(c, "k_group_post");
-      k_group_post<<<c->num_sms * 16, 256, 0, c->stream>>>(a);
-    }
-    KLU_TRY(check_launch("k_group_post"));
-  } else if (a.num_items > 0) {
+  if (a.num_items > 0) {
     // shared memory: the largest window of the batch, capped (runs beyond the cap take the slow path)
     const int kMaxWinBytes = 64 << 10;
     KLU_CUDA(cudaFuncSetAttribute(k_frame_groups, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxWinBytes));  // per device

@@ -268,59 +268,19 @@ __global__ void __launch_bounds__(256) k_gp_lat_scan(const int32_t* cnt, const i
   __shared__ long long carry_s;
   const int l = blockIdx.x;
   const int i0 = seg_off[l], n = seg_off[l + 1] - i0;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   if (tid == 0) carry_s = 0;
   __syncthreads();
   for (int tile = 0; tile < n; tile += 256) {
     const int i = tile + tid;
     const long long c = i < n ? cnt[i0 + i] : 0;
-    long long x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const long long y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    long long add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
+    const long long pre = cta_exclusive_scan<long long, 256>(c, warp_sum, carry_s);
     if (i < n) {
-      if (MODE == 0) out32[i0 + i] = base32[l] + (int32_t)(add + x - c);
-      else out64[i0 + i] = add + x - c;
+      if (MODE == 0) out32[i0 + i] = base32[l] + (int32_t)(pre);
+      else out64[i0 + i] = pre;
     }
-    __syncthreads();
-    if (tid == 255) carry_s = add + x;
-    __syncthreads();
   }
   if (tid == 0 && MODE == 1) lat_tot[l] = carry_s;
-}
-
-// exclusive scan of L per-lattice totals (single block), in place: tot[l] -> base, tot[L] = sum
-__global__ void __launch_bounds__(1024) k_gp_scan_tot(long long* tot, int L) {
-  __shared__ long long warp_sum[32];
-  __shared__ long long carry_s;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) carry_s = 0;
-  __syncthreads();
-  for (int tile = 0; tile < L; tile += 1024) {
-    const int i = tile + tid;
-    const long long c = i < L ? tot[i] : 0;
-    long long x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const long long y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    long long add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    __syncthreads();
-    if (i < L) tot[i] = add + x - c;
-    if (tid == 1023) carry_s = add + x;
-    __syncthreads();
-  }
-  if (tid == 0) tot[L] = carry_s;
 }
 
 // lattice-local int64 offsets -> global: off[i] += base[l]; also the closing entry
@@ -466,25 +426,14 @@ __global__ void __launch_bounds__(256) k_gp_frame_counts(GP a) {
   const int l = blockIdx.x;
   const int n = a.fr_base[l + 1] - a.fr_base[l];
   int32_t* cnt = a.fr_cnt + a.fr_base[l];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   if (tid == 0) carry_s = 0;
   __syncthreads();
   for (int tile = 0; tile < n; tile += 256) {
     const int i = tile + tid;
-    int x = i < n ? cnt[i] : 0;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    int add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (i < n) cnt[i] = add + x;
-    __syncthreads();
-    if (tid == 255) carry_s = add + x;
-    __syncthreads();
+    const int v = i < n ? cnt[i] : 0;
+    const int pre = cta_exclusive_scan<int, 256>(v, warp_sum, carry_s);
+    if (i < n) cnt[i] = pre + v;
   }
 }
 
@@ -849,11 +798,7 @@ int pack_and_upload_gpu(klu_ctx* c, const klu_lattices* in) {
     k_gp_lat_scan<1><<<L, 256, 0, c->stream>>>(a.counts, a.s_off, nullptr, nullptr, a.band_off, a.lat_tot);
   }
   KLU_TRY(check_launch("k_gp_lat_scan(band)"));
-  {
-    KLU_LAUNCH(c, "k_gp_scan_tot");
-    k_gp_scan_tot<<<1, 1024, 0, c->stream>>>(a.lat_tot, L);
-  }
-  KLU_TRY(check_launch("k_gp_scan_tot(band)"));
+  KLU_TRY(scan_counts(c, a.lat_tot, 0, L, a.lat_tot, "k_gp_scan_tot"));
   {
     KLU_LAUNCH(c, "k_gp_add_base");
     k_gp_add_base<<<dim3(L, st_tiles), 256, 0, c->stream>>>(a.band_off, a.s_off, a.lat_tot, L, a.band_off + S);

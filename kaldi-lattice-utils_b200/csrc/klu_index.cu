@@ -100,27 +100,15 @@ __global__ void __launch_bounds__(256) k_count_scan(IndexArgs a) {
   __shared__ int carry_s;
   const int l = a.l0 + blockIdx.x;
   const int e0 = a.b.e_off[l], e1 = a.b.e_off[l + 1];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   const int T = a.b.fr_base[l + 1] - a.b.fr_base[l] - 1;  // frames of the utterance
   if (tid == 0) carry_s = 0;
   __syncthreads();
   for (int tile = e0; tile < e1; tile += 256) {
     const int e = tile + tid;
     const int c = e < e1 ? arc_entry_count(a, e, T) : 0;
-    int x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    int add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (e < e1) a.arc_ent_off[e] = add + x - c;
-    __syncthreads();
-    if (tid == 255) carry_s = add + x;
-    __syncthreads();
+    const int pre = cta_exclusive_scan<int, 256>(c, warp_sum, carry_s);
+    if (e < e1) a.arc_ent_off[e] = pre;
   }
   if (tid == 0) a.ent_cnt[l] = carry_s;
 }
@@ -292,26 +280,14 @@ __global__ void __launch_bounds__(256) k_reduce_offsets(ReduceArgs a) {
   const int n = a.ent_cnt[l];
   const int ntiles = (n + 255) >> 8;
   int32_t* cnt = a.tile_heads + tile_slot(a, l, 0);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   if (tid == 0) carry_s = 0;
   __syncthreads();
   for (int t0 = 0; t0 < ntiles; t0 += 256) {
     const int t = t0 + tid;
     const int v = t < ntiles ? cnt[t] : 0;
-    int x = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    int add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (t < ntiles) cnt[t] = add + x - v;
-    __syncthreads();
-    if (tid == 255) carry_s = add + x;
-    __syncthreads();
+    const int pre = cta_exclusive_scan<int, 256>(v, warp_sum, carry_s);
+    if (t < ntiles) cnt[t] = pre;
   }
   if (tid == 0) a.rcnt[l] = carry_s;
 }
@@ -441,35 +417,6 @@ __global__ void __launch_bounds__(256) k_reduce(ReduceArgs a) {
     }
     __syncthreads();  // the staging arrays are rewritten by the next tile
   }
-}
-
-// res_off[l] = sum_{l' < l} rcnt[l'] (single block, L is small next to the arcs)
-// off[l0] must already hold the running total of the previous chunks.
-__global__ void __launch_bounds__(1024) k_scan_counts(const int32_t* cnt, int l0, int L, int64_t* off) {
-  __shared__ long long warp_sum[32];
-  __shared__ long long carry_s;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) carry_s = off[l0];
-  __syncthreads();
-  for (int tile = l0; tile < L; tile += 1024) {
-    const int i = tile + tid;
-    const long long c = i < L ? cnt[i] : 0;
-    long long x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const long long y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    long long add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (i < L) off[i] = add + x - c;
-    __syncthreads();
-    if (tid == 1023) carry_s = add + x;
-    __syncthreads();
-  }
-  if (tid == 0) off[L] = carry_s;
 }
 
 // The order sort looks at the high half of the f64 keys only (32-bit keys: half the radix
@@ -631,15 +578,7 @@ __global__ void __launch_bounds__(256) k_utt_tasks(UttArgs a) {
     chunk = __shfl_sync(0xffffffffu, chunk, 0);
     const long long tc = t_begin + (long long)chunk;
     if (tc >= t_end) break;
-    {  // lattice of the chunk's first item: last l with res_off[l] <= tc
-      int lo = a.l0, hi = a.l0 + a.nl - 1;
-      while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (a.res_off[mid] <= tc) lo = mid;
-        else hi = mid - 1;
-      }
-      l = lo;
-    }
+    l = last_le(a.res_off, a.l0, a.l0 + a.nl - 1, tc);  // lattice of the chunk's first item
     for (long long t = tc; t < min(tc + 4, t_end); ++t) {
       while (a.res_off[l + 1] <= t) ++l;
       const int slot = (int)(t - a.res_off[l]);
@@ -1001,11 +940,7 @@ int run_index_tool(klu_ctx* c, int tool, const klu_opts* o) {
       u.vbwd = a.vbwd;
       u.best = a.best;
       u.beam = a.beam;
-      {
-        KLU_LAUNCH(c, "k_scan_counts");
-        k_scan_counts<<<1, 1024, 0, c->stream>>>(r.rcnt, l0, l1, c->d_res[5].as<int64_t>());
-      }
-      KLU_TRY(check_launch("k_scan_counts"));
+      KLU_TRY(scan_counts(c, r.rcnt, l0, l1, c->d_res[5].as<int64_t>(), "k_scan_counts"));
       u.res_off = c->d_res[5].as<int64_t>();
       const int grid = std::max(1, c->num_sms * 4);
       KLU_TRY(c->d_alpha2.reserve(sizeof(double) * (size_t)grid * 8 * (size_t)u.max_states));
@@ -1070,11 +1005,7 @@ int run_index_tool(klu_ctx* c, int tool, const klu_opts* o) {
       }
       KLU_TRY(check_launch("k_seg_radix_sort(order)"));
     }
-    {
-      KLU_LAUNCH(c, "k_scan_counts");
-      k_scan_counts<<<1, 1024, 0, c->stream>>>(r.rcnt, l0, l1, c->d_res[5].as<int64_t>());
-    }
-    KLU_TRY(check_launch("k_scan_counts"));
+    KLU_TRY(scan_counts(c, r.rcnt, l0, l1, c->d_res[5].as<int64_t>(), "k_scan_counts"));
     if (single_chunk) {
       KLU_TRY(grow_results(chunk_cap));
     } else {

@@ -68,33 +68,6 @@ __global__ void __launch_bounds__(128) k_len_emit(LenArgs a) {
   if (lane == 0) a.cnt[l] = n;
 }
 
-__global__ void __launch_bounds__(1024) k_len_scan(const int32_t* cnt, int L, int64_t* off) {
-  __shared__ long long warp_sum[32];
-  __shared__ long long carry_s;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) carry_s = 0;
-  __syncthreads();
-  for (int tile = 0; tile < L; tile += 1024) {
-    const int i = tile + tid;
-    const long long c = i < L ? cnt[i] : 0;
-    long long x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const long long y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    long long add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (i < L) off[i] = add + x - c;
-    __syncthreads();
-    if (tid == 1023) carry_s = add + x;
-    __syncthreads();
-  }
-  if (tid == 0) off[L] = carry_s;
-}
-
 __global__ void __launch_bounds__(128) k_len_gather(const int64_t* ent_base, const int32_t* cnt, const int64_t* res_off,
                                                     const unsigned long long* key_a, const unsigned long long* key_b,
                                                     const unsigned char* where, int32_t* o_len, float* o_logp, int L) {
@@ -173,14 +146,10 @@ int run_length_dist(klu_ctx* c, const klu_opts* o) {
   ss.hi_bit = 64;
   {
     KLU_LAUNCH(c, "k_seg_radix_sort");
-    seg_sort_launch(ss, L, c->num_sms, c->stream);
+    seg_sort_launch(ss, L, c->stream);
   }
   KLU_TRY(check_launch("k_seg_radix_sort(length dist)"));
-  {
-    KLU_LAUNCH(c, "k_len_scan");
-    k_len_scan<<<1, 1024, 0, c->stream>>>(a.cnt, L, c->d_res[5].as<int64_t>());
-  }
-  KLU_TRY(check_launch("k_len_scan"));
+  KLU_TRY(scan_counts(c, a.cnt, 0, L, c->d_res[5].as<int64_t>(), "k_len_scan"));
   {
     KLU_LAUNCH(c, "k_len_gather");
     k_len_gather<<<(L * 32 + 127) / 128, 128, 0, c->stream>>>(a.ent_base, a.cnt, c->d_res[5].as<int64_t>(), ss.key_a, ss.key_b,

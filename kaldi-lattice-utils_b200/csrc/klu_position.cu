@@ -169,26 +169,14 @@ __global__ void __launch_bounds__(256) k_tile_prefix(const int64_t* base, const 
   const long long n = n64 ? n64[l] : (long long)n32[l];
   const int ntiles = (int)((n + 255) >> 8);
   int32_t* cnt = tiles + tile_slot(base, l, l_first, 0);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   if (tid == 0) carry_s = 0;
   __syncthreads();
   for (int t0 = 0; t0 < ntiles; t0 += 256) {
     const int t = t0 + tid;
     const int v = t < ntiles ? cnt[t] : 0;
-    int x = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    int add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (t < ntiles) cnt[t] = add + x - v;
-    __syncthreads();
-    if (tid == 255) carry_s = add + x;
-    __syncthreads();
+    const int pre = cta_exclusive_scan<int, 256>(v, warp_sum, carry_s);
+    if (t < ntiles) cnt[t] = pre;
   }
   if (tid == 0) total[l] = carry_s;
 }
@@ -250,26 +238,14 @@ __global__ void __launch_bounds__(256) k_pos_cell_offsets(PosArgs a) {
   __shared__ long long carry_s;
   const int l = blockIdx.x;
   const int e0 = a.b.e_off[l], n = a.ngroups[l];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   if (tid == 0) carry_s = 0;
   __syncthreads();
   for (int tile = 0; tile < n; tile += 256) {
     const int i = tile + tid;
     const long long c = i < n ? a.g_celloff[e0 + i] : 0;
-    long long x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const long long y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    long long add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (i < n) a.g_celloff[e0 + i] = (int32_t)min(add + x - c, (long long)0x7fffffff);
-    __syncthreads();
-    if (tid == 255) carry_s = add + x;
-    __syncthreads();
+    const long long pre = cta_exclusive_scan<long long, 256>(c, warp_sum, carry_s);
+    if (i < n) a.g_celloff[e0 + i] = (int32_t)min(pre, (long long)0x7fffffff);
   }
   if (tid == 0) a.lat_cells[l] = carry_s;
 }
@@ -312,12 +288,7 @@ __global__ void __launch_bounds__(256) k_pos_tile_groups(PosArgs a) {
   const long long ntiles = (ncells + 255) >> 8;
   for (long long t = (long long)blockIdx.y * blockDim.x + threadIdx.x; t < ntiles; t += (long long)gridDim.y * blockDim.x) {
     const long long first = t << 8;
-    int lo = 0, hi = ng - 1;  // last group with celloff <= first
-    while (lo < hi) {
-      const int mid = (lo + hi + 1) >> 1;
-      if ((long long)celloff[mid] <= first) lo = mid;
-      else hi = mid - 1;
-    }
+    const int lo = last_le(celloff, 0, ng - 1, first);  // last group with celloff <= first
     a.tile_group[tile_slot(a.cell_base, l, a.l0, (int)t)] = lo;
   }
 }
@@ -480,34 +451,6 @@ __global__ void __launch_bounds__(256) k_pos_compact(PosArgs a) {
     }
     __syncthreads();
   }
-}
-
-// res_off[l] = rows of the lattices before l (single block); off[l0] holds the previous chunks' total
-__global__ void __launch_bounds__(1024) k_pos_scan_counts(const int32_t* cnt, int l0, int L, int64_t* off) {
-  __shared__ long long warp_sum[32];
-  __shared__ long long carry_s;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) carry_s = off[l0];
-  __syncthreads();
-  for (int tile = l0; tile < L; tile += 1024) {
-    const int i = tile + tid;
-    const long long c = i < L ? cnt[i] : 0;
-    long long x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const long long y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    long long add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (i < L) off[i] = add + x - c;
-    __syncthreads();
-    if (tid == 1023) carry_s = add + x;
-    __syncthreads();
-  }
-  if (tid == 0) off[L] = carry_s;
 }
 
 // The order sort of the position index runs on the high half of the f64 keys only (32-bit
@@ -936,11 +879,7 @@ int run_position_tool(klu_ctx* c, int tool, const klu_opts* o) {
       }
       KLU_TRY(check_launch("k_seg_radix_sort(order)"));
     }
-    {
-      KLU_LAUNCH(c, "k_scan_counts");
-      k_pos_scan_counts<<<1, 1024, 0, c->stream>>>(a.rcnt, l0, l1, c->d_res[5].as<int64_t>());
-    }
-    KLU_TRY(check_launch("k_scan_counts"));
+    KLU_TRY(scan_counts(c, a.rcnt, l0, l1, c->d_res[5].as<int64_t>(), "k_scan_counts"));
     {
       int64_t upto = 0;
       KLU_CUDA(cudaMemcpyAsync(&upto, c->d_res[5].as<int64_t>() + l1, sizeof(int64_t), cudaMemcpyDeviceToHost,

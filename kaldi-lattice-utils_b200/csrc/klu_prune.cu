@@ -182,7 +182,7 @@ __global__ void __launch_bounds__(256) k_prune_scan(PruneArgs a) {
   __shared__ int warp_sum[8];
   __shared__ int carry_s;
   const int l = blockIdx.x;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   for (int which = 0; which < 2; ++which) {
     int* flags = which == 0 ? a.arc_keep : a.state_keep;
     const int i0 = which == 0 ? a.b.e_off[l] : a.b.s_off[l];
@@ -193,21 +193,9 @@ __global__ void __launch_bounds__(256) k_prune_scan(PruneArgs a) {
     for (int tile = i0; tile < i1; tile += 256) {
       const int i = tile + tid;
       const int c = i < i1 ? flags[i] : 0;
-      int x = c;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const int y = __shfl_up_sync(0xffffffffu, x, o);
-        if (lane >= o) x += y;
-      }
-      if (lane == 31) warp_sum[warp] = x;
-      __syncthreads();
-      int add = carry_s;
-      for (int w = 0; w < warp; ++w) add += warp_sum[w];
+      const int pre = cta_exclusive_scan<int, 256>(c, warp_sum, carry_s);
       // exclusive rank, sign bit marks "dropped"
-      if (i < i1) flags[i] = c ? (add + x - c) : -1;
-      __syncthreads();
-      if (tid == 255) carry_s = add + x;
-      __syncthreads();
+      if (i < i1) flags[i] = c ? pre : -1;
     }
     if (tid == 0) (which == 0 ? a.arc_cnt : a.state_cnt)[l] = carry_s;
   }
@@ -261,33 +249,6 @@ __global__ void __launch_bounds__(256) k_prune_emit(PruneArgs a) {
     a.o_fg[os] = keep_final ? g : INFINITY;
     a.o_fa[os] = keep_final ? w : INFINITY;
   }
-}
-
-__global__ void __launch_bounds__(1024) k_scan_counts32(const int32_t* cnt, int L, int64_t* off) {
-  __shared__ long long warp_sum[32];
-  __shared__ long long carry_s;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) carry_s = 0;
-  __syncthreads();
-  for (int tile = 0; tile < L; tile += 1024) {
-    const int i = tile + tid;
-    const long long c = i < L ? cnt[i] : 0;
-    long long x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const long long y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    long long add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (i < L) off[i] = add + x - c;
-    __syncthreads();
-    if (tid == 1023) carry_s = add + x;
-    __syncthreads();
-  }
-  if (tid == 0) off[L] = carry_s;
 }
 
 // ----------------------------------------------------------- lattice-prune-arcs ---
@@ -577,11 +538,7 @@ int run_prune_arcs(klu_ctx* c, const klu_opts* o) {
     k_prune_scan<<<L, 256, 0, c->stream>>>(a);
   }
   KLU_TRY(check_launch("k_prune_scan"));
-  {
-    KLU_LAUNCH(c, "k_scan_counts");
-    k_scan_counts32<<<1, 1024, 0, c->stream>>>(a.arc_cnt, L, c->d_res[5].as<int64_t>());
-  }
-  KLU_TRY(check_launch("k_scan_counts"));
+  KLU_TRY(scan_counts(c, a.arc_cnt, 0, L, c->d_res[5].as<int64_t>(), "k_scan_counts"));
   {
     KLU_LAUNCH(c, "k_pa_emit");
     k_pa_emit<<<dim3(L, tiles), 256, 0, c->stream>>>(a, p);
@@ -683,11 +640,7 @@ int run_prune_dyn_beam(klu_ctx* c, const klu_opts* o) {
     k_prune_scan<<<L, 256, 0, c->stream>>>(a);
   }
   KLU_TRY(check_launch("k_prune_scan"));
-  {
-    KLU_LAUNCH(c, "k_scan_counts");
-    k_scan_counts32<<<1, 1024, 0, c->stream>>>(a.arc_cnt, L, c->d_res[5].as<int64_t>());
-  }
-  KLU_TRY(check_launch("k_scan_counts"));
+  KLU_TRY(scan_counts(c, a.arc_cnt, 0, L, c->d_res[5].as<int64_t>(), "k_scan_counts"));
   {
     KLU_LAUNCH(c, "k_prune_emit");
     k_prune_emit<<<dim3(L, tiles), 256, 0, c->stream>>>(a);

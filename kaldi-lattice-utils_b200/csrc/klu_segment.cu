@@ -107,13 +107,7 @@ __global__ void __launch_bounds__(256) k_sg_bucket_offsets(BatchView b, const in
   const int slot = blockIdx.x * blockDim.x + threadIdx.x;
   int mine = 0;
   if (slot < num_slots) {
-    int lo = 0, hi = b.L - 1;  // lattice of the slot
-    while (lo < hi) {
-      const int mid = (lo + hi + 1) >> 1;
-      if (slot_base[mid] <= slot) lo = mid;
-      else hi = mid - 1;
-    }
-    const int l = lo;
+    const int l = last_le(slot_base, 0, b.L - 1, slot);  // lattice of the slot
     const unsigned int k = (unsigned int)(slot - slot_base[l]);
     const int e0 = b.e_off[l], n = b.e_off[l + 1] - e0;
     const unsigned int* key = (where[l] ? key_b : key_a) + e0;
@@ -265,26 +259,14 @@ __global__ void __launch_bounds__(256) k_sg_dense_offsets(SegArgs a) {
   __shared__ int carry_s;
   const int l = blockIdx.x;
   const int slot0 = a.slot_base[l], nslots = a.slot_base[l + 1] - slot0;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   if (tid == 0) carry_s = 0;
   __syncthreads();
   for (int base = 0; base < nslots; base += 256) {
     const int i = base + tid;
     const int c = i < nslots ? a.slot_cnt[slot0 + i] : 0;
-    int x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    int add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (i < nslots) a.slot_dense[slot0 + i] = add + x - c;
-    __syncthreads();
-    if (tid == 255) carry_s = add + x;
-    __syncthreads();
+    const int pre = cta_exclusive_scan<int, 256>(c, warp_sum, carry_s);
+    if (i < nslots) a.slot_dense[slot0 + i] = pre;
   }
   if (tid == 0) a.rcnt[l] = carry_s;
 }
@@ -348,34 +330,6 @@ __global__ void __launch_bounds__(256) k_sg_order_fixup(SegFixArgs a) {
       ++j;
     }
   }
-}
-
-// res_off[l] = entries of the lattices before l (single block)
-__global__ void __launch_bounds__(1024) k_sg_scan_counts(const int32_t* cnt, int L, int64_t* off) {
-  __shared__ long long warp_sum[32];
-  __shared__ long long carry_s;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) carry_s = 0;
-  __syncthreads();
-  for (int tile = 0; tile < L; tile += 1024) {
-    const int i = tile + tid;
-    const long long c = i < L ? cnt[i] : 0;
-    long long x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const long long y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    long long add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (i < L) off[i] = add + x - c;
-    __syncthreads();
-    if (tid == 1023) carry_s = add + x;
-    __syncthreads();
-  }
-  if (tid == 0) off[L] = carry_s;
 }
 
 struct SegGatherArgs {
@@ -645,11 +599,7 @@ int run_segment_buckets(klu_ctx* c, const klu_opts* o, bool* done) {
     k_sg_order_fixup<<<(unsigned int)((int64_t)L * tiles), 256, 0, c->stream>>>(f);
   }
   KLU_TRY(check_launch("k_order_fixup"));
-  {
-    KLU_LAUNCH(c, "k_scan_counts");
-    k_sg_scan_counts<<<1, 1024, 0, c->stream>>>(a.rcnt, L, c->d_res[5].as<int64_t>());
-  }
-  KLU_TRY(check_launch("k_scan_counts"));
+  KLU_TRY(scan_counts(c, a.rcnt, 0, L, c->d_res[5].as<int64_t>(), "k_scan_counts"));
   // result columns: at most one entry per arc
   KLU_TRY(c->d_res[0].reserve(4 * E1));
   KLU_TRY(c->d_res[1].reserve(4 * E1));

@@ -241,11 +241,9 @@ static inline void seg_sort_launch_w(const SegSortArgsT<K>& a, int nseg, cudaStr
 }
 
 template <typename K>
-static inline void seg_sort_launch(const SegSortArgsT<K>& a, int nseg, int num_sms, cudaStream_t stream) {
-  (void)num_sms;
+static inline void seg_sort_launch(const SegSortArgsT<K>& a, int nseg, cudaStream_t stream) {
   if (nseg <= 0) return;
-  static const bool narrow_only = getenv("KLU_SORT_8BIT") != nullptr;
-  const int w = narrow_only ? 8 : seg_sort_digit_bits(a.hi_bit - a.lo_bit);
+  const int w = seg_sort_digit_bits(a.hi_bit - a.lo_bit);
   if (w == 9) seg_sort_launch_w<K, 9>(a, nseg, stream);
   else if (w == 10) seg_sort_launch_w<K, 10>(a, nseg, stream);
   else seg_sort_launch_w<K, 8>(a, nseg, stream);
@@ -280,27 +278,15 @@ struct MsWork {
 static __global__ void __launch_bounds__(1024) k_ms_plan(const int32_t* seg_cnt, int nseg, int32_t* tile_first) {
   __shared__ int warp_sum[32];
   __shared__ int carry_s;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   if (tid == 0) carry_s = 0;
   __syncthreads();
   for (int base = 0; base < nseg; base += 1024) {
     const int i = base + tid;
     const int n = i < nseg ? seg_cnt[i] : 0;
     const int c = n <= 1 ? 0 : (n + kMsTile - 1) / kMsTile;
-    int x = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    int add = carry_s;
-    for (int w = 0; w < warp; ++w) add += warp_sum[w];
-    if (i < nseg) tile_first[i] = add + x - c;
-    __syncthreads();
-    if (tid == 1023) carry_s = add + x;
-    __syncthreads();
+    const int pre = cta_exclusive_scan<int, 1024>(c, warp_sum, carry_s);
+    if (i < nseg) tile_first[i] = pre;
   }
   if (tid == 0) tile_first[nseg] = carry_s;
 }
@@ -603,7 +589,7 @@ static inline int seg_sort_launch(klu_ctx* c, const SegSortArgsT<K>& a, int nseg
   const int64_t avg = total / nseg;
   const bool multi = multi_only || (!single_only && avg >= 2 * kMsTile && (nseg < c->num_sms * 8 || avg >= 64 * kMsTile));
   if (!multi) {
-    seg_sort_launch(a, nseg, c->num_sms, c->stream);
+    seg_sort_launch(a, nseg, c->stream);
     return 0;
   }
   return seg_sort_multi(a, nseg, total, c->num_sms, c->stream, c->d_sortws, &c->launches);

@@ -10,13 +10,13 @@
 //                  lattice that DisambiguateStateInputSequenceLength
 //                  (fstext/fstext-utils2.h:109-215) would materialise.
 //
-// One warp owns one (lattice, direction) work item, pulled from a queue sorted by
-// descending arc count.  Inside a level the warp is split into 32/G groups of G
-// lanes; a group owns one state and pulls over its incoming (forward) or outgoing
-// (backward) arcs with coalesced 16-byte record loads, reduces max and sum-exp
-// with shuffles, and lane 0 of the group writes the f64 score.  State scores live
-// in global memory and are re-read through L1 (same-SM producer/consumer, ordered
-// by __syncwarp between levels).
+// Log sweeps: a warp takes 32/G lattices of one direction from a queue sorted by
+// descending arc count, and a tile of G lanes sweeps one of them level by level
+// (log_sweep_tiles).  A tile stages a batch of a level's arc records in shared
+// memory, forms every arc's exp term around one shared reference point, and adds
+// each state's terms with a few lanes.  State scores are written to global memory
+// and to a per-tile shared-memory ring of recent states; the far end of an arc is
+// read from the ring when it is still there, else gathered from global memory.
 #include <stdlib.h>
 
 #include "klu_common.cuh"
@@ -123,7 +123,7 @@ __device__ __noinline__ double sweep_state_exact(const SweepArgs& a, int l, int 
 // dependent chain; what the machine can overlap is OTHER lattices).
 //
 // Inside a level a tile cuts the states into batches of <= G states and
-// <= 16 G arcs.  The arcs of a batch are one contiguous run of 16-byte records
+// <= kCap = 8 G arcs.  The arcs of a batch are one contiguous run of 16-byte records
 // (in_rec is sorted by destination, out_rec by source): the tile's lanes stream
 // them, each lane turns its arcs into exp(score[other] - cost - ref) and parks the
 // term in shared memory.  `ref` is the score of the previous batch's first state: a
@@ -318,264 +318,6 @@ __global__ void __launch_bounds__(128) k_log_sweeps(const __grid_constant__ Swee
     const int first = (unit - (fwd || !a.do_fwd ? 0 : per_dir)) * NG;
     if (fwd) log_sweep_tiles<G, true, BEAM>(a, first, lane, xwarp, rwarp);
     else log_sweep_tiles<G, false, BEAM>(a, first, lane, xwarp, rwarp);
-    __syncwarp();
-  }
-}
-
-// ---------------------------------------------------------------------------
-// The same sweep with the record staging moved to the copy engine and taken off the
-// dependency chain (sm_90+ bulk copies, "TMA 1D"): a batch's records are one contiguous run
-// of 16-byte structs, so ONE lane of the tile issues ONE cp.async.bulk for the whole run and
-// an mbarrier counts its bytes in -- no per-lane copy loop, no address arithmetic per
-// record.  And because the extent of the NEXT batch depends on the lattice structure only
-// (CSR offsets), its copy is issued before the current batch is processed: two record
-// buffers per tile, the fetch of batch k+1 overlaps the exp/log work of batch k instead of
-// standing between two levels of the chain.
-__device__ __forceinline__ unsigned int smem_addr(const void* p) { return (unsigned int)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_addr(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned int bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, unsigned int bytes, unsigned long long* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   smem_addr(dst)),
-               "l"(src), "r"(bytes), "r"(smem_addr(bar))
-               : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(unsigned long long* bar, unsigned int parity) {
-  unsigned int ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(smem_addr(bar)), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-// (four tiles per warp at G = 8: a 64-entry ring keeps the static shared memory under 48 KB)
-__host__ __device__ constexpr int sweep_ring2(int G) { return G >= 16 ? 128 : 64; }
-
-template <int G, int CPL, bool FWD, bool BEAM>
-__device__ void log_sweep_tiles2(const SweepArgs& a, int first, int lane, double2* xwarp, double* rwarp,
-                                 unsigned long long* bars, unsigned int& phase) {
-  constexpr int kCap = CPL * G;
-  constexpr int NG = 32 / G;
-  constexpr int kRing = sweep_ring2(G);
-  constexpr int kLog2G = G == 32 ? 5 : G == 16 ? 4 : G == 8 ? 3 : G == 4 ? 2 : 1;
-  const BatchView& b = a.b;
-  const int gi = lane / G, sl = lane % G;
-  const unsigned int gmask = (G == 32 ? 0xffffffffu : ((1u << G) - 1u)) << (gi * G);
-  double2* xb0 = xwarp + gi * kCap;             // record / term buffers of this tile: [buffer][tile][kCap]
-  double2* xb1 = xwarp + (NG + gi) * kCap;
-  unsigned long long* bar = bars + 2 * gi;      // one mbarrier per buffer
-  double* ring = rwarp + gi * kRing;
-  const int4* rec = FWD ? b.in_rec : b.out_rec;
-  const int* off = FWD ? b.in_off : b.out_off;
-  double* score = FWD ? a.alpha : a.beta;
-  bool done = first + gi >= b.L;
-  const int l = done ? 0 : b.order[first + gi];
-  const int s_begin = b.s_off[l];
-  if (!done && s_begin == b.s_off[l + 1]) done = true;
-  const int* lv = b.lvl_start + b.lvl_off[l];
-  const int nl = b.lvl_off[l + 1] - b.lvl_off[l] - 1;
-  double ref = 0.0;
-  int j = FWD ? 1 : nl - 1;
-  if (FWD && !done)
-    for (int s = lv[0] + sl; s < lv[1]; s += G) {
-      const double v = (s == s_begin) ? 0.0 : neg_inf();
-      score[s] = v;
-      ring[s & (kRing - 1)] = v;
-    }
-  if (!done && (FWD ? j >= nl : j < 0)) done = true;
-  int a0 = 0, a1 = 0, s0 = 0;
-  int wide = 0x7fffffff;  // backward: first state of the nearest level above wider than kRing (see log_sweep_tiles)
-  if (!done) {
-    s0 = a0 = lv[j];
-    a1 = lv[j + 1];
-  }
-  __syncwarp();
-  // ---- extent of the batch at (done, s0, a1): the longest prefix of the level's remaining states whose
-  //      arcs fit the buffer; every lane keeps its state's arc range, the tile its base / count / arcs
-  int o_lo, o_hi, base, c, nb;
-  auto extent = [&](bool dn, int st, int lim, int& x_lo, int& x_hi, int& x_base, int& x_c, int& x_nb) {
-    const int idx = st + sl;
-    x_lo = 0;
-    x_hi = 0;
-    if (!dn) {
-      x_lo = off[min(idx, lim)];
-      x_hi = off[min(idx + 1, lim)];
-    }
-    x_base = __shfl_sync(0xffffffffu, x_lo, 0, G);
-    const unsigned int fit = __ballot_sync(0xffffffffu, !dn && idx < lim && x_hi - x_base <= kCap) & gmask;
-    x_c = __popc(fit);
-    const int o_last = __shfl_sync(0xffffffffu, x_hi, max(x_c - 1, 0), G);
-    x_nb = x_c > 0 ? o_last - x_base : 0;
-  };
-  auto issue = [&](bool dn, int x_base, int x_nb, int buf) {
-    if (!dn && x_nb > 0 && sl == 0) {
-      fence_proxy_async();  // the buffer's last use (generic-proxy reads / writes) is ordered before the copy
-      mbar_expect_tx(bar + buf, 16u * (unsigned int)x_nb);
-      bulk_g2s(buf ? xb1 : xb0, rec + x_base, 16u * (unsigned int)x_nb, bar + buf);
-    }
-  };
-  extent(done, s0, a1, o_lo, o_hi, base, c, nb);
-  int cur = 0;
-  issue(done, base, nb, cur);
-  while (!__all_sync(0xffffffffu, done)) {
-    // ---- where the NEXT batch starts, its extent, its copy
-    bool n_done = done;
-    int n_j = j, n_a0 = a0, n_a1 = a1, n_s0 = s0, n_wide = wide;
-    if (!done) {
-      n_s0 = s0 + (c > 0 ? c : 1);
-      if (n_s0 >= a1) {
-        if (!FWD && a1 - a0 > kRing) n_wide = a0;
-        n_j = j + (FWD ? 1 : -1);
-        if (FWD ? n_j >= nl : n_j < 0) {
-          n_done = true;
-        } else {
-          n_s0 = n_a0 = lv[n_j];
-          n_a1 = lv[n_j + 1];
-        }
-      }
-    }
-    int n_lo, n_hi, n_base, n_c, n_nb;
-    extent(n_done, n_s0, n_a1, n_lo, n_hi, n_base, n_c, n_nb);
-    issue(n_done, n_base, n_nb, cur ^ 1);
-    if (!n_done && n_c > 0) {  // pull the records a few levels ahead into L2
-      const int pf = n_base + n_nb + kCap + sl * 8;
-      if (sl * 8 < n_nb && pf < b.E) asm volatile("prefetch.global.L2 [%0];" ::"l"(rec + pf));
-    }
-    // ---- the current batch's records have landed?
-    double2* xbuf = cur ? xb1 : xb0;
-    if (!done && nb > 0) {
-      while (!mbar_try_wait(bar + cur, (phase >> (2 * gi + cur)) & 1u)) {
-      }
-      phase ^= 1u << (2 * gi + cur);
-    }
-    __syncwarp();
-    // ---- cost and exp term of the lane's own arcs; scores of far ends gathered asynchronously
-    unsigned int pending = 0;
-    {
-      int it = 0;
-      for (int i = sl; i < nb; i += G, ++it) {
-        const int4 r = *reinterpret_cast<const int4*>(xbuf + i);
-        double cost = rec_cost(r, a.cp);
-        if (BEAM && sweep_arc_pruned<FWD, BEAM>(a, l, base + i, r)) cost = pos_inf();
-        const int t = r.x;
-        if (FWD ? (t >= a1 - kRing) : (t < min(a0 + kRing, wide))) {
-          xbuf[i].x = fast_exp(ring[t & (kRing - 1)] - cost - ref);
-        } else {
-          xbuf[i].x = cost;
-          cp_async8(&xbuf[i].y, score + t);
-          pending |= 1u << it;
-        }
-      }
-    }
-    if (__any_sync(0xffffffffu, pending != 0)) {
-      cp_async_wait_all();
-      int it = 0;
-      for (int i = sl; i < nb; i += G, ++it) {
-        if ((pending >> it) & 1u) {
-          const double2 v = xbuf[i];
-          xbuf[i].x = fast_exp(v.y - v.x - ref);
-        }
-      }
-    }
-    __syncwarp();
-    // ---- G / pow2ceil(c) lanes per state add its terms, then fold across those lanes
-    const int sh = c <= 1 ? kLog2G : kLog2G - (32 - __clz(c - 1));
-    const int gp = 1 << sh;
-    const int st = sl >> sh, sub = sl & (gp - 1);
-    const int lo = __shfl_sync(0xffffffffu, o_lo, st, G) - base, hi = __shfl_sync(0xffffffffu, o_hi, st, G) - base;
-    double sum = 0.0;
-    if (st < c)
-      for (int i = lo + sub; i < hi; i += gp) sum += xbuf[i].x;
-#pragma unroll
-    for (int o = G / 2; o > 0; o >>= 1) {
-      const double v = __shfl_xor_sync(0xffffffffu, sum, o, G);
-      if (o < gp) sum += v;
-    }
-    bool bad = false;
-    double val = 0.0;
-    if (st < c && sub == 0) {
-      const int s = s0 + st;
-      double fin = neg_inf();
-      if (!FWD) {
-        const double fc = final_cost(b.fin_g[s], b.fin_a[s], a.cp);
-        if (fc < pos_inf() && !(BEAM && final_pruned(a, l, s, fc))) {
-          fin = -fc;
-          sum += fast_exp(fin - ref);
-        }
-      }
-      const int terms = hi - lo + (fin > neg_inf() ? 1 : 0);
-      if (terms <= 2) {
-        // one or two terms: exactly Kaldi's LogAdd, so chains and diamonds reproduce the reference bit for bit
-        val = fin;
-        for (int i = lo; i < hi; ++i) {
-          const int4 r = __ldg(rec + base + i);
-          double x = score[r.x] - rec_cost(r, a.cp);
-          if (BEAM && sweep_arc_pruned<FWD, BEAM>(a, l, base + i, r)) x = neg_inf();
-          val = log_add(val, x);
-        }
-      } else if (sum >= 1e-280 && sum <= 1e280) {
-        val = ref + fast_log(sum);
-      } else {
-        bad = true;
-      }
-      if (bad) val = sweep_state_exact<FWD, BEAM>(a, l, s);
-      score[s] = val;
-      ring[s & (kRing - 1)] = val;
-    }
-    if (!done && c == 0 && sl == 0) {  // a single state with more arcs than the tile stages
-      val = sweep_state_exact<FWD, BEAM>(a, l, s0);
-      score[s0] = val;
-      ring[s0 & (kRing - 1)] = val;
-    }
-    const double v0 = __shfl_sync(0xffffffffu, val, 0, G);
-    if (!done && v0 > neg_inf() && v0 < pos_inf()) ref = v0;
-    // ---- the prefetched batch becomes the current one
-    done = n_done;
-    j = n_j;
-    a0 = n_a0;
-    a1 = n_a1;
-    s0 = n_s0;
-    wide = n_wide;
-    o_lo = n_lo;
-    o_hi = n_hi;
-    base = n_base;
-    c = n_c;
-    nb = n_nb;
-    cur ^= 1;
-    __syncwarp();
-  }
-}
-
-template <int G, int CPL, bool BEAM, int MB>
-__global__ void __launch_bounds__(128, MB) k_log_sweeps2(const __grid_constant__ SweepArgs a) {
-  constexpr int NG = 32 / G;
-  __shared__ __align__(16) double2 xs[4][2 * NG * CPL * G];  // per warp: two buffers x NG tiles x CPL * G records
-  __shared__ double rings[4][NG * sweep_ring2(G)];
-  __shared__ __align__(8) unsigned long long bars[4][2 * NG];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  if (lane < 2 * NG) mbar_init(&bars[warp][lane], 1);
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  fence_proxy_async();
-  __syncwarp();
-  unsigned int phase = 0;  // bit 2 * tile + buffer: parity the next wait on that barrier looks for
-  const int per_dir = (a.b.L + NG - 1) / NG;
-  const int nunits = per_dir * (a.do_fwd + a.do_bwd);
-  for (;;) {
-    int unit = 0;
-    if (lane == 0) unit = atomicAdd(a.counter, 1);
-    unit = __shfl_sync(0xffffffffu, unit, 0);
-    if (unit >= nunits) break;
-    const bool fwd = a.do_fwd && unit < per_dir;
-    const int first = (unit - (fwd || !a.do_fwd ? 0 : per_dir)) * NG;
-    if (fwd) log_sweep_tiles2<G, CPL, true, BEAM>(a, first, lane, xs[warp], rings[warp], bars[warp], phase);
-    else log_sweep_tiles2<G, CPL, false, BEAM>(a, first, lane, xs[warp], rings[warp], bars[warp], phase);
     __syncwarp();
   }
 }
@@ -791,12 +533,7 @@ __global__ void __launch_bounds__(kBandThreads) k_banded_alpha(SweepArgs a, doub
             const int nz = r.w != 0 ? 1 : 0;
             bool dead = plo < 0 || pw <= 0;
             if (BEAM && !dead) {
-              int lo = 0, hi = take - 1;  // the arc's destination: last k with ss_arc[k] <= e
-              while (lo < hi) {
-                const int mid = (lo + hi + 1) >> 1;
-                if (ss_arc[mid] - e_base <= i) lo = mid;
-                else hi = mid - 1;
-              }
+              const int lo = last_le(ss_arc, 0, take - 1, e_base + i);  // the arc's destination: last k with ss_arc[k] <= e
               dead = arc_pruned(a, l, r.x, s0 + lo, r);
             }
             sa_cost[i] = rec_cost(r, a.cp);
@@ -807,12 +544,7 @@ __global__ void __launch_bounds__(kBandThreads) k_banded_alpha(SweepArgs a, doub
         __syncthreads();
         const long long c0 = ss_cell[0], c1 = ss_cell[take];
         for (long long cell = c0 + tid; cell < c1; cell += kBandThreads) {
-          int lo = 0, hi = take - 1;  // last k with ss_cell[k] <= cell
-          while (lo < hi) {
-            const int mid = (lo + hi + 1) >> 1;
-            if (ss_cell[mid] <= cell) lo = mid;
-            else hi = mid - 1;
-          }
+          const int lo = last_le(ss_cell, 0, take - 1, cell);  // last k with ss_cell[k] <= cell
           const int len = ss_lo[lo] + (int)(cell - ss_cell[lo]);
           LogSumRun acc;
           if (staged) {
@@ -941,30 +673,10 @@ int run_log_sweeps(klu_ctx* c, const CostParams& cp, bool use_beam, float beam) 
   }
   const int units = 2 * ((c->L + 32 / G - 1) / (32 / G));
   const int grid = sweep_grid(c, units);
-  // KLU_SWEEP_V2=1: the bulk-copy (cp.async.bulk + mbarrier, next batch prefetched) variant.  Measured
-  // slower than the cp.async one on 10 k c2 lattices (8.5-8.9 ms against 6.3 ms, profiles/r2_sweeps_v2.md):
-  // a batch's records are <= 2 KB, the bulk copy's issue-to-arrival latency is longer than one batch's
-  // math, and two record buffers per tile cost residency.  Kept selectable as a cross-check.
-  // KLU_SWEEP_CPL / KLU_SWEEP_MB: its records per lane per batch / resident CTAs the registers are cut for.
-  static const bool v1 = getenv("KLU_SWEEP_V2") == nullptr;
-  static const int cpl = getenv("KLU_SWEEP_CPL") ? atoi(getenv("KLU_SWEEP_CPL")) : 8;
-  static const int mb = getenv("KLU_SWEEP_MB") ? atoi(getenv("KLU_SWEEP_MB")) : 7;
   {
     KLU_LAUNCH(c, "k_log_sweeps");
-    if (v1 || G < 8) {
-      KLU_DISPATCH_G(G, if (use_beam) k_log_sweeps<kG, true><<<grid, 128, 0, c->stream>>>(a);
-                     else k_log_sweeps<kG, false><<<grid, 128, 0, c->stream>>>(a));
-    } else {
-      // (records per lane per batch, resident CTAs per SM the register budget is cut for): tuning knobs
-#define KLU_SWEEP2(CPL, MB)                                                                                      \
-  KLU_DISPATCH_G(G, if (use_beam) k_log_sweeps2<(kG < 8 ? 8 : kG), CPL, true, MB><<<grid, 128, 0, c->stream>>>(a); \
-                 else k_log_sweeps2<(kG < 8 ? 8 : kG), CPL, false, MB><<<grid, 128, 0, c->stream>>>(a))
-      if (cpl == 4 && mb >= 7) { KLU_SWEEP2(4, 7); }
-      else if (cpl == 4) { KLU_SWEEP2(4, 5); }
-      else if (mb >= 7) { KLU_SWEEP2(8, 7); }
-      else { KLU_SWEEP2(8, 5); }
-#undef KLU_SWEEP2
-    }
+    KLU_DISPATCH_G(G, if (use_beam) k_log_sweeps<kG, true><<<grid, 128, 0, c->stream>>>(a);
+                   else k_log_sweeps<kG, false><<<grid, 128, 0, c->stream>>>(a));
   }
   KLU_TRY(check_launch("k_log_sweeps"));
   {

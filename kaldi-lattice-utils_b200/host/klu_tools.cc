@@ -146,7 +146,6 @@ struct Batch {
     v.fin_graph = fin_graph.data();
     v.fin_acoustic = fin_acoustic.data();
     v.fin_dur = fin_dur.data();
-    if (getenv("KLU_PLAIN_UPLOAD")) return v;
     const size_t E = src.size(), S = fin_graph.size(), nl = lats.size();
     num_arcs_.assign(S, 0);
     dur8_.resize(E);

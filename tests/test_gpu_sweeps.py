@@ -1,13 +1,13 @@
 """The sweep kernels of klu_sweep.cu per state, at every instantiation and branch.
 
-The log sweeps (`k_log_sweeps<G>`, and `k_log_sweeps2<G, CPL>` under KLU_SWEEP_V2=1) stage
-the arcs of a batch of states in shared memory (kCap arcs per tile), keep recent state
-scores in a ring (kRing slots) and switch on the number of terms of a state (one or two:
-Kaldi's LogAdd; more: a streaming sum around a shared reference point, redone exactly when
-it leaves [1e-280, 1e280]; more arcs than the tile stages: the exact one-lane sum).  Every
-one of those switches moves with G.  The builders below put states exactly at, below and
-above each switch for a given (G, kCap, kRing) and every state's alpha and beta is compared
-with the oracle's ComputeLatticeAlphasAndBetas restatement.
+The log sweeps (`k_log_sweeps<G>`) stage the arcs of a batch of states in shared memory
+(kCap arcs per tile), keep recent state scores in a ring (kRing slots) and switch on the
+number of terms of a state (one or two: Kaldi's LogAdd; more: a streaming sum around a
+shared reference point, redone exactly when it leaves [1e-280, 1e280]; more arcs than the
+tile stages: the exact one-lane sum).  Every one of those switches moves with G.  The
+builders below put states exactly at, below and above each switch for a given (G, kCap,
+kRing) and every state's alpha and beta is compared with the oracle's
+ComputeLatticeAlphasAndBetas restatement.
 
 Also here: the tropical sweeps at each `pick_group` width (through lattice-prune-dyn-beam and
 lattice-best-path2), the pieces of `k_banded_alpha` (through the position tools), and the
@@ -16,7 +16,6 @@ import os
 import re
 import shutil
 import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -30,13 +29,9 @@ PKG = os.path.join(ROOT, "kaldi-lattice-utils_b200")
 
 # ---- the constants of klu_sweep.cu, restated ---------------------------------------------------
 # k_log_sweeps<G>:         kCap = kSweepCapPerLane * G = 8 G arcs per batch, kRing = sweep_ring(G)
-# k_log_sweeps2<G, CPL>:   kCap = CPL * G (KLU_SWEEP_CPL, default 8), kRing = sweep_ring2(G);
-#                          run_log_sweeps takes it only for G >= 8 (below: k_log_sweeps<G>)
 # k_banded_alpha:          pieces of <= kBandStates = 128 states and <= kBandArcs = 768 arcs
 # k_trop_sweeps<G>:        G = pick_group(arcs / states of the batch)
-SWEEP_V2 = os.environ.get("KLU_SWEEP_V2") is not None
-SWEEP_CPL = int(os.environ.get("KLU_SWEEP_CPL", "8"))
-GROUPS = (8, 16, 32) if SWEEP_V2 else (2, 4, 8, 16, 32)
+GROUPS = (2, 4, 8, 16, 32)
 BAND_STATES, BAND_ARCS = 128, 768
 
 
@@ -44,14 +39,8 @@ def sweep_ring(g):
     return 128 if g >= 8 else 32
 
 
-def sweep_ring2(g):
-    return 128 if g >= 16 else 64
-
-
 def sweep_consts(g):
     """(kCap, kRing) of the kernel run_log_sweeps launches at lane width g."""
-    if SWEEP_V2 and g >= 8:
-        return SWEEP_CPL * g, sweep_ring2(g)
     return 8 * g, sweep_ring(g)
 
 
@@ -425,22 +414,7 @@ def test_automatic_width_at_scale(klu, ora, engine, monkeypatch):
         check_batch(ora, batch, engine.fetch_fwd_bwd(), flags, "auto G=16 %r" % flags, only=sample)
 
 
-# ---- 3. the bulk-copy variant in a child process -------------------------------------------------
-@pytest.mark.skipif(SWEEP_V2, reason="already the child")
-@pytest.mark.parametrize("cpl", [4, 8])
-def test_bulk_copy_sweeps(tmp_path, cpl):
-    """KLU_SWEEP_V2=1 selects k_log_sweeps2 (read once per process, hence the child): the log
-    sweep tests above at G = 8, 16, 32 with its own staging cap CPL * G and ring sweep_ring2(G)."""
-    env = dict(os.environ, KLU_SWEEP_V2="1", KLU_SWEEP_CPL=str(cpl))
-    log = tmp_path / ("sweeps_v2_cpl%d.log" % cpl)
-    with open(str(log), "w") as f:
-        rc = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-m", "gpu", "-x", "-q",
-                             "-k", "log_sweeps or two_term", "-p", "no:cacheprovider"],
-                            env=env, cwd=ROOT, stdout=f, stderr=subprocess.STDOUT, timeout=900).returncode
-    assert rc == 0, "sweep tests failed with KLU_SWEEP_V2=1 KLU_SWEEP_CPL=%d:\n%s" % (cpl, log.read_text()[-3000:])
-
-
-# ---- 4. tropical sweeps at every pick_group width ------------------------------------------------
+# ---- 3. tropical sweeps at every pick_group width ------------------------------------------------
 def fanout_lattice(klu, rng, key, width, nlev, deg, ties):
     """start -> nlev levels of `width` states -> final.  Every state of a level but the last
     sends `deg` arcs to the next level (parallel arcs), the first of them to the state with
@@ -503,7 +477,7 @@ def test_tropical_sweeps_each_width(klu, ora, engine, target, group):
             assert abs(bp[l][1] - cost) <= 1e-4 * max(1.0, abs(cost))
 
 
-# ---- 5. k_banded_alpha pieces ---------------------------------------------------------------
+# ---- 4. k_banded_alpha pieces ---------------------------------------------------------------
 def band_lattice(klu, rng, key, width=None, in_counts=None):
     """start -> a level of `width` states -> (optionally) states with the given in-arc counts
     from that level -> final.  Labels on the first two hops only: at most 3 distinct lengths."""
@@ -573,7 +547,7 @@ def test_banded_alpha_pieces(klu, ora, engine, monkeypatch, flags):
                 assert abs(dict(g)[wd] - v) <= 1e-4, "position-post %s position %d word %d" % (lat.key, p, wd)
 
 
-# ---- 6. fast_exp / fast_log / log_add on the device ---------------------------------------------
+# ---- 5. fast_exp / fast_log / log_add on the device ---------------------------------------------
 PROBE = r"""
 #include <stdio.h>
 #include <vector>
