@@ -102,9 +102,7 @@ struct BatchView {
   const int64_t* band_off;   // [S+1] offsets into the (state,len) band arrays
   const int32_t* order;      // [L] lattices by descending arc count (work queue order)
   const int32_t* fr_base;    // [L+1] first slot of each lattice in fr_off (num_frames + 1 slots per lattice)
-  const int64_t* fr_off;     // per (lattice, frame): first entry of the frame in frame_arc
-  const int32_t* frame_arc;  // per frame: out-order arc ids (global) of the word arcs alive in it, sorted by
-                             // (word, arc); bit 31 marks the first arc of every word group
+  const int64_t* fr_off;     // per (lattice, frame): first arc x frame instance of the frame
 };
 
 struct KernelStat {
@@ -156,6 +154,7 @@ struct klu_ctx {
   std::vector<int64_t> h_frame_res_off;      // [L+1] frame-post output rows per lattice (static per batch)
   int32_t fr_items = 0;                      // frame-post work items (runs of frames)
   int32_t fr_max_window = 0;                 // largest arc window of a run of frames
+  bool fr_id16 = true;                       // frame index instance ids are 16-bit (else 32-bit)
   int32_t max_label = 0, max_time = 0, max_len = 0, max_indeg = 0, max_outdeg = 0, max_states = 0;
   int32_t max_span = 0;  // longest arc in frames (time[dst] - time[src])
   double avg_deg = 0;
@@ -164,7 +163,7 @@ struct klu_ctx {
   // ---- device: packed batch ----
   klu::DevBuf d_s_off, d_e_off, d_lvl_off, d_lvl_start, d_in_rec, d_out_rec, d_in_off, d_out_off, d_out_src,
       d_in2out, d_old2new, d_out_orig, d_fin_g, d_fin_a, d_time, d_orig, d_level, d_band_lo, d_band_off, d_order, d_fr_base, d_fr_off, d_frame_arc,
-      d_fr_item, d_fr_gloc, d_fr_res_off, d_fr_gword, d_fr_gstart, d_fr_gframe, d_fr_run_lo, d_fr_run_hi, d_fr_tarc, d_fr_tlabel, d_fr_seg, d_tile_heads, d_sg_meta, d_sg_boff, d_sg_perm, d_sortws;
+      d_fr_item, d_fr_gloc, d_fr_res_off, d_fr_gword, d_fr_gstart, d_fr_gframe, d_fr_run_lo, d_fr_run_hi, d_fr_tarc, d_fr_item_lat, d_fr_seg, d_tile_heads, d_sg_meta, d_sg_boff, d_sg_perm, d_sortws;
   // ---- device: per-run state ----
   klu::DevBuf d_alpha, d_beta, d_total, d_totfwd, d_counter, d_filter;
   klu::DevBuf d_vfwd, d_vbwd, d_best;  // tropical sweeps
@@ -216,7 +215,11 @@ int run_segment_buckets(klu_ctx* c, const klu_opts* o, bool* done);
 // klu_position.cu: lattice-word-index-position, lattice-to-word-position-post, lattice-best-path2
 int run_position_tool(klu_ctx* c, int tool, const klu_opts* o);
 // klu_frame.cu
-int build_frame_groups(klu_ctx* c);  // pack time: (frame, word)-sorted instances, head bits, output offsets
+int build_frame_groups(klu_ctx* c);  // pack time: (frame, word)-sorted instances, window offsets, output offsets
+// The packers' part of the frame index: per out-order arc its first frame if it is a word arc
+// that spans one, else frame_time_tail(c->max_time), into the buffer reserve_frame_time_keys returns.
+uint32_t frame_time_tail(int32_t max_time);
+int reserve_frame_time_keys(klu_ctx* c, uint32_t** keys);
 int run_frame_post(klu_ctx* c, const klu_opts* o);
 // klu_prune.cu
 int run_prune_dyn_beam(klu_ctx* c, const klu_opts* o);

@@ -239,7 +239,6 @@ klu::BatchView klu_ctx::view() const {
   v.order = d_order.as<int32_t>();
   v.fr_base = d_fr_base.as<int32_t>();
   v.fr_off = d_fr_off.as<int64_t>();
-  v.frame_arc = d_frame_arc.as<int32_t>();
   return v;
 }
 
@@ -319,7 +318,7 @@ int klu_destroy(klu_ctx* c) {
   cudaStreamSynchronize(c->stream);
   DevBuf* bufs[] = {&c->d_s_off, &c->d_e_off, &c->d_lvl_off, &c->d_lvl_start, &c->d_in_rec, &c->d_out_rec,
                     &c->d_in_off, &c->d_out_off, &c->d_out_src, &c->d_out_orig, &c->d_in2out, &c->d_old2new, &c->d_fin_g, &c->d_fin_a,
-                    &c->d_time, &c->d_orig, &c->d_level, &c->d_band_lo, &c->d_band_off, &c->d_order, &c->d_fr_base, &c->d_fr_off, &c->d_frame_arc, &c->d_fr_item, &c->d_fr_gloc, &c->d_fr_res_off, &c->d_fr_gword, &c->d_fr_gstart, &c->d_fr_gframe, &c->d_fr_run_lo, &c->d_fr_run_hi, &c->d_fr_tarc, &c->d_fr_tlabel, &c->d_fr_seg, &c->d_tile_heads, &c->d_sg_meta, &c->d_sg_boff, &c->d_sg_perm, &c->d_sortws, &c->d_alpha, &c->d_beta,
+                    &c->d_time, &c->d_orig, &c->d_level, &c->d_band_lo, &c->d_band_off, &c->d_order, &c->d_fr_base, &c->d_fr_off, &c->d_frame_arc, &c->d_fr_item, &c->d_fr_gloc, &c->d_fr_res_off, &c->d_fr_gword, &c->d_fr_gstart, &c->d_fr_gframe, &c->d_fr_run_lo, &c->d_fr_run_hi, &c->d_fr_tarc, &c->d_fr_item_lat, &c->d_fr_seg, &c->d_tile_heads, &c->d_sg_meta, &c->d_sg_boff, &c->d_sg_perm, &c->d_sortws, &c->d_alpha, &c->d_beta,
                     &c->d_total, &c->d_totfwd, &c->d_counter, &c->d_filter, &c->d_vfwd, &c->d_vbwd, &c->d_best,
                     &c->d_alpha2, &c->d_flush};
   char_release(c);

@@ -7,10 +7,11 @@
 //
 // Which (frame, word) groups exist, which arcs feed each of them and how many rows
 // every frame emits depends only on labels and state times, not on the weights.
-// So klu_load() builds that structure ONCE per batch (build_frame_groups): the arcs
-// numbered by start time, the arc x frame instances of a lattice sorted by (frame,
-// word, arc), a head bit on the first instance of every group, and the dense output
-// offset of every frame.  A run is then the log sweeps and two kernels:
+// So klu_load() builds that structure ONCE per batch (build_frame_groups): the word
+// arcs numbered by start time, the arc x frame instances of a lattice sorted by (frame,
+// word, arc), each naming its arc by its offset in its run's window, the first
+// instance of every group, and the dense output offset of every frame.  A run is then
+// the log sweeps and two kernels:
 //   k_frame_groups  one CTA per run of kFramesPerItem frames: the posterior
 //                   exp(fw[u] + bw[v] - cost - total) of every arc of the run's
 //                   window into shared memory (f64; exp(-700) ~ 1e-304 is the
@@ -49,13 +50,16 @@ struct FrameArgs {
   const double* beta;
   const double* total;
   const int32_t* item_base;  // [L+1] first work item of each lattice
+  const int32_t* item_lat;   // [num_items] lattice of each work item
   int num_items;
   const int64_t* gloc;       // per frame slot: lattice-local first output row (T+1 per lattice)
   const int64_t* res_off;    // [L+1] first output row of each lattice
   const int32_t* gwords;     // word of every (frame, word) group, in pre-order row order (static)
   const uint32_t* gstart;    // [rows + 1] first instance of every group (static)
-  const int4* tarc;          // [E] arcs in START-TIME order: {src, dst, graph bits, acoustic bits} (static)
-  const int32_t* tlabel;     // [E] their labels; frame_arc holds indices into this order
+  const int4* tarc;          // [E] arcs in START-TIME order: {src, dst, graph bits, acoustic bits} (static);
+                             // per lattice the word arcs that span a frame come first
+  const void* ids;           // [instances] per instance: its arc's time-order index minus its run's run_lo,
+                             // uint16_t when every window is shorter than 65536 arcs, else uint32_t (static)
   const int32_t* run_lo;     // per work item (run of frames): smallest / largest time-order arc index among
   const int32_t* run_hi;     // its instances (static); the arcs in between are the run's "window"
   int win_cap;               // window entries that fit the dynamic shared memory
@@ -68,30 +72,27 @@ __device__ __forceinline__ float inv_ord_f32(unsigned int u) {
   return __uint_as_float(b);
 }
 
+// the record of a word arc of the time-order copy as rec_cost reads it (any non-zero label
+// adds the insertion penalty; every arc an instance names has one)
+__device__ __forceinline__ int4 word_rec(const int4& t) { return make_int4(t.y, t.z, t.w, 1); }
+
 // fw[u] + bw[next] - (float)(g + a), latbin/lattice-to-word-frame-post.cc:102-104
 __device__ __forceinline__ double arc_value(const FrameArgs& a, int j) {  // j: time-order arc index
   const int4 t = __ldg(a.tarc + j);
-  const int4 r = make_int4(t.y, t.z, t.w, __ldg(a.tlabel + j));
-  return __dadd_rn(__dadd_rn(a.alpha[t.x], a.beta[t.y]), -rec_cost(r, a.cp));
+  return __dadd_rn(__dadd_rn(a.alpha[t.x], a.beta[t.y]), -rec_cost(word_rec(t), a.cp));
 }
 
-// Exact log-posterior of the group that ENDS at instance `iend` of a frame's list
-// (walks back to the group's head): max first, then libm exp / log.
-__device__ __noinline__ double exact_group_logp(const FrameArgs& a, const int32_t* fa, int iend, double total) {
+// Exact log-posterior of the group of instances [i0, i1) of a run whose window starts at
+// wlo: max first, then libm exp / log, adding from the group's last instance down.
+template <typename Id>
+__device__ __forceinline__ double exact_group_logp(const FrameArgs& a, const Id* ids, uint32_t i0, uint32_t i1, int wlo,
+                                                double total) {
   double m = neg_inf();
-  for (int q = iend;; --q) {
-    const unsigned int w = (unsigned int)fa[q];
-    m = fmax(m, arc_value(a, (int)(w & 0x7fffffffu)));
-    if (w >> 31) break;
-  }
+  for (uint32_t i = i1; i-- > i0;) m = fmax(m, arc_value(a, wlo + (int)ids[i]));
   if (!(m > neg_inf())) return neg_inf();
   if (m == pos_inf()) return pos_inf();
   double s = 0.0;
-  for (int q = iend;; --q) {
-    const unsigned int w = (unsigned int)fa[q];
-    s += exp(arc_value(a, (int)(w & 0x7fffffffu)) - m);
-    if (w >> 31) break;
-  }
+  for (uint32_t i = i1; i-- > i0;) s += exp(arc_value(a, wlo + (int)ids[i]) - m);
   return (m + log(s)) - total;
 }
 
@@ -170,24 +171,30 @@ __device__ void warp_sort_rows_global(float* logp, int32_t* word, int n, int lan
 
 
 // Fused arc posteriors + group sums for one run of kFramesPerItem frames per CTA.
-// With the arcs numbered by start time (a copy made at pack time), the word arcs alive
-// in a run of frames are a contiguous index range -- the run's window.  Phase 1 computes the posterior of
-// every arc of the window into shared memory (coalesced record reads, one exp per arc;
-// windows of neighbouring runs overlap by the arcs that span the boundary, ~1/8 extra);
-// phase 2 adds each (frame, word) group's posteriors, one thread per group, from shared
-// memory.  No per-arc posterior array in HBM, no dependent global gathers.  Runs whose window does not fit
-// (very long arcs) take the posteriors from alpha/beta directly, instance by instance.
+// With the word arcs numbered by start time (a copy made at pack time), the word arcs
+// alive in a run of frames are a contiguous index range -- the run's window.  Phase 1
+// computes the posterior of every arc of the window into shared memory (coalesced record
+// reads, one exp per arc; windows of neighbouring runs overlap by the arcs that span the
+// boundary, ~1/8 extra); phase 2 adds each (frame, word) group's posteriors, one thread
+// per group, from shared memory, reading every instance as its arc's offset in the window
+// (Id: 16 bits when all windows of the batch allow it).  No per-arc posterior array in
+// HBM, no dependent global gathers.  Runs whose window does not fit (very long arcs) take
+// the posteriors from alpha/beta directly, instance by instance.
+template <typename Id>
 __global__ void __launch_bounds__(128) k_frame_groups(const __grid_constant__ FrameArgs a) {
   extern __shared__ double s_post[];
   const BatchView& b = a.b;
   const int item = blockIdx.x;
-  const int l = last_le(a.item_base, 0, b.L - 1, item);  // lattice of this item
-  const int T = b.fr_base[l + 1] - b.fr_base[l] - 1;
+  const int l = __ldg(a.item_lat + item);
+  const int fb = b.fr_base[l];
+  const int T = b.fr_base[l + 1] - fb - 1;
   const int k0 = (item - a.item_base[l]) * kFramesPerItem;
   const int k1 = min(T, k0 + kFramesPerItem);
-  const int64_t* gl = a.gloc + b.fr_base[l];
-  const int64_t row0 = a.res_off[l] + gl[k0], row1 = a.res_off[l] + gl[k1];
-  if (row0 == row1) return;
+  const int64_t* gl = a.gloc + fb;
+  const int64_t row0 = a.res_off[l] + gl[k0];
+  const int nrows = (int)(gl[k1] - gl[k0]);  // rows of the run, addressed from row0 below
+  if (nrows == 0) return;
+  const Id* ids = static_cast<const Id*>(a.ids);
   const int wlo = a.run_lo[item], whi = a.run_hi[item];
   const bool windowed = whi - wlo < a.win_cap;
   const double total = a.total[l];
@@ -200,26 +207,22 @@ __global__ void __launch_bounds__(128) k_frame_groups(const __grid_constant__ Fr
     // dependent chain (offset -> id -> shared-memory posterior), find them there
     const int pl = threadIdx.x - 96;
     const char* q = reinterpret_cast<const char*>(a.gstart + row0);
-    const int64_t qb = (row1 - row0 + 1) * 4;
-    for (int64_t off = pl * 128; off < qb; off += 32 * 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(q + off));
-    const uint32_t ilo = __ldg(a.gstart + row0), ihi = __ldg(a.gstart + row1);
-    q = reinterpret_cast<const char*>(b.frame_arc + ilo);
-    const int64_t ib = (int64_t)(ihi - ilo) * 4;
+    const int qb = (nrows + 1) * 4;
+    for (int off = pl * 128; off < qb; off += 32 * 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(q + off));
+    const uint32_t ilo = __ldg(a.gstart + row0), ihi = __ldg(a.gstart + row0 + nrows);
+    q = reinterpret_cast<const char*>(ids + ilo);
+    const int64_t ib = (int64_t)(ihi - ilo) * sizeof(Id);
     for (int64_t off = pl * 128; off < ib; off += 32 * 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(q + off));
   }
   if (windowed) {
-    // four arcs per thread and trip: their record, label and score loads go out together
+    // four arcs per thread and trip: their record and score loads go out together
     for (int j0 = wlo + threadIdx.x; j0 <= whi; j0 += 4 * blockDim.x) {
       int4 t[4];
-      int lab[4];
       double al[4], be[4];
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
         const int j = j0 + u * blockDim.x;
-        if (j <= whi) {
-          t[u] = __ldg(a.tarc + j);
-          lab[u] = __ldg(a.tlabel + j);
-        }
+        if (j <= whi) t[u] = __ldg(a.tarc + j);
       }
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
@@ -232,10 +235,7 @@ __global__ void __launch_bounds__(128) k_frame_groups(const __grid_constant__ Fr
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
         const int j = j0 + u * blockDim.x;
-        if (j <= whi) {
-          const int4 r = make_int4(t[u].y, t[u].z, t[u].w, lab[u]);
-          s_post[j - wlo] = lab[u] != 0 ? fast_exp(__dadd_rn(__dadd_rn(al[u], be[u]), -rec_cost(r, a.cp)) - total) : 0.0;
-        }
+        if (j <= whi) s_post[j - wlo] = fast_exp(__dadd_rn(__dadd_rn(al[u], be[u]), -rec_cost(word_rec(t[u]), a.cp)) - total);
       }
     }
     __syncthreads();
@@ -246,23 +246,22 @@ __global__ void __launch_bounds__(128) k_frame_groups(const __grid_constant__ Fr
   // summed afterwards, long ones side by side.  A group is always added up by one
   // thread in instance order, so which thread does it cannot change the result.
   // (trip count uniform across a warp: the list push below is a warp-wide ballot)
-  for (int64_t g0 = row0 + threadIdx.x; g0 - (threadIdx.x & 31) < row1; g0 += 2 * blockDim.x) {
+  for (int g0 = threadIdx.x; g0 - (int)(threadIdx.x & 31) < nrows; g0 += 2 * blockDim.x) {
     uint32_t i0[2], i1[2];
     double sum[2] = {0.0, 0.0};
     bool defer[2] = {false, false};
 #pragma unroll
     for (int v = 0; v < 2; ++v) {
-      const int64_t g = g0 + v * blockDim.x;
-      i0[v] = g < row1 ? __ldg(a.gstart + g) : 0u;
-      i1[v] = g < row1 ? __ldg(a.gstart + g + 1) : 0u;
+      const int g = g0 + v * blockDim.x;
+      i0[v] = g < nrows ? __ldg(a.gstart + row0 + g) : 0u;
+      i1[v] = g < nrows ? __ldg(a.gstart + row0 + g + 1) : 0u;
     }
     if (windowed) {
       int e[2][4];
 #pragma unroll
       for (int v = 0; v < 2; ++v)
 #pragma unroll
-        for (int u = 0; u < 4; ++u)
-          e[v][u] = i0[v] + u < i1[v] ? (int)((unsigned int)__ldg(b.frame_arc + i0[v] + u) & 0x7fffffffu) - wlo : -1;
+        for (int u = 0; u < 4; ++u) e[v][u] = i0[v] + u < i1[v] ? (int)__ldg(ids + i0[v] + u) : -1;
 #pragma unroll
       for (int v = 0; v < 2; ++v) {
 #pragma unroll
@@ -276,26 +275,24 @@ __global__ void __launch_bounds__(128) k_frame_groups(const __grid_constant__ Fr
           base = __shfl_sync(0xffffffffu, base, 0);
           const int slot = base + __popc(m & ((1u << lane) - 1u));
           if (is_long && slot < kLongCap) {
-            s_long[slot] = (int)(g0 + v * blockDim.x - row0);
+            s_long[slot] = g0 + v * blockDim.x;
             defer[v] = true;
           }
         }
         if (!defer[v])
-          for (uint32_t i = i0[v] + 4; i < i1[v]; ++i)
-            sum[v] += s_post[(int)((unsigned int)__ldg(b.frame_arc + i) & 0x7fffffffu) - wlo];
+          for (uint32_t i = i0[v] + 4; i < i1[v]; ++i) sum[v] += s_post[__ldg(ids + i)];
       }
     } else {
 #pragma unroll
       for (int v = 0; v < 2; ++v)
-        for (uint32_t i = i0[v]; i < i1[v]; ++i)
-          sum[v] += fast_exp(arc_value(a, (int)((unsigned int)__ldg(b.frame_arc + i) & 0x7fffffffu)) - total);
+        for (uint32_t i = i0[v]; i < i1[v]; ++i) sum[v] += fast_exp(arc_value(a, wlo + (int)__ldg(ids + i)) - total);
     }
 #pragma unroll
     for (int v = 0; v < 2; ++v) {
-      const int64_t g = g0 + v * blockDim.x;
-      if (g < row1 && !defer[v]) {
-        const double lp = sum[v] >= 1e-280 ? fast_log(sum[v]) : exact_group_logp(a, b.frame_arc, i1[v] - 1, total);
-        a.o_logp[g] = (float)lp + 0.0f;  // -0.0 and +0.0 compare equal in the reference's sort
+      const int g = g0 + v * blockDim.x;
+      if (g < nrows && !defer[v]) {
+        const double lp = sum[v] >= 1e-280 ? fast_log(sum[v]) : exact_group_logp(a, ids, i0[v], i1[v], wlo, total);
+        a.o_logp[row0 + g] = (float)lp + 0.0f;  // -0.0 and +0.0 compare equal in the reference's sort
       }
     }
   }
@@ -303,20 +300,20 @@ __global__ void __launch_bounds__(128) k_frame_groups(const __grid_constant__ Fr
   __syncthreads();
   const int nlong = min(s_nlong, kLongCap);
   for (int k = threadIdx.x; k < nlong; k += blockDim.x) {
-    const int64_t g = row0 + s_long[k];
-    const uint32_t i0 = __ldg(a.gstart + g), i1 = __ldg(a.gstart + g + 1);
+    const int g = s_long[k];
+    const uint32_t i0 = __ldg(a.gstart + row0 + g), i1 = __ldg(a.gstart + row0 + g + 1);
     double sum = 0.0;
     uint32_t i = i0;
     for (; i + 4 <= i1; i += 4) {  // four ids in flight
       int e[4];
 #pragma unroll
-      for (int u = 0; u < 4; ++u) e[u] = (int)((unsigned int)__ldg(b.frame_arc + i + u) & 0x7fffffffu) - wlo;
+      for (int u = 0; u < 4; ++u) e[u] = __ldg(ids + i + u);
 #pragma unroll
       for (int u = 0; u < 4; ++u) sum += s_post[e[u]];
     }
-    for (; i < i1; ++i) sum += s_post[(int)((unsigned int)__ldg(b.frame_arc + i) & 0x7fffffffu) - wlo];
-    const double lp = sum >= 1e-280 ? fast_log(sum) : exact_group_logp(a, b.frame_arc, i1 - 1, total);
-    a.o_logp[g] = (float)lp + 0.0f;
+    for (; i < i1; ++i) sum += s_post[__ldg(ids + i)];
+    const double lp = sum >= 1e-280 ? fast_log(sum) : exact_group_logp(a, ids, i0, i1, wlo, total);
+    a.o_logp[row0 + g] = (float)lp + 0.0f;
   }
 }
 
@@ -416,7 +413,7 @@ __global__ void __launch_bounds__(kFrameWarps * 32, 8) k_frame_order(const __gri
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const BatchView& b = a.b;
   for (int item = blockIdx.x * kFrameWarps + warp; item < a.num_items; item += gridDim.x * kFrameWarps) {
-    const int l = last_le(a.item_base, 0, b.L - 1, item);  // lattice of this item
+    const int l = __ldg(a.item_lat + item);
     const int T = b.fr_base[l + 1] - b.fr_base[l] - 1;
     const int k0 = (item - a.item_base[l]) * kFramesPerItem;
     const int k1 = min(T, k0 + kFramesPerItem);
@@ -464,9 +461,11 @@ struct GroupArgs {
   const unsigned int *val_a, *val_b;
   const unsigned char* where;
   int k32;                   // the (frame, word) keys fit 32 bits: the key buffers hold unsigned ints
-  int32_t* frame_arc;
+  void* ids;                 // FrameArgs::ids
+  int id16;                  // ... as uint16_t (else uint32_t)
   int32_t* frame_cnt;        // per frame slot: groups in the frame
   const int32_t* item_base;
+  int32_t* item_lat;
   int num_items;
   int64_t* gloc;
   int32_t* lat_cnt;
@@ -479,18 +478,24 @@ struct GroupArgs {
   const int64_t* arc_base;   // [L] = e_off as 64-bit segment bases
   int32_t* rank_of;          // [E] out-order arc -> time-order index (global)
   int4* tarc;
-  int32_t* tlabel;
 };
 
-// grid (L, tiles): sort input for the time order: key = start frame, val = out-order arc (lattice-local)
+__device__ __forceinline__ int arc_frames(const BatchView& b, int e, int T, int* first) {
+  const int4 r = b.out_rec[e];
+  if (r.w == 0) return 0;
+  const int fa = max(b.time[b.out_src[e]], 0), fb = min(b.time[r.x], T);
+  *first = fa;
+  return fb > fa ? fb - fa : 0;
+}
+
+// grid (L, tiles): sort values for the time order, val = out-order arc (lattice-local); the keys
+// are the packer's (frame_time_keys)
 __global__ void __launch_bounds__(256) k_fg_time_keys(GroupArgs a) {
   const LatTile lt = lat_tile();  // CTAs that run together share lattices (L2 locality)
   const int l = lt.l;
   const int e0 = a.b.e_off[l], e1 = a.b.e_off[l + 1];
-  for (int e = e0 + lt.tile * blockDim.x + threadIdx.x; e < e1; e += lt.tiles * blockDim.x) {
-    reinterpret_cast<unsigned int*>(a.key)[e] = (unsigned int)max(a.b.time[a.b.out_src[e]], 0);  // 32-bit keys
+  for (int e = e0 + lt.tile * blockDim.x + threadIdx.x; e < e1; e += lt.tiles * blockDim.x)
     a.val[e] = (unsigned int)(e - e0);
-  }
 }
 
 // grid (L, tiles): the time-ordered arc copy and the inverse permutation
@@ -503,22 +508,14 @@ __global__ void __launch_bounds__(256) k_fg_time_copy(GroupArgs a) {
     const int e = e0 + (int)val[j - e0];
     const int4 r = a.b.out_rec[e];
     a.tarc[j] = make_int4(a.b.out_src[e], r.x, r.y, r.z);
-    a.tlabel[j] = r.w;
     a.rank_of[e] = j;
   }
 }
 
-__device__ __forceinline__ int arc_frames(const BatchView& b, int e, int T, int* first) {
-  const int4 r = b.out_rec[e];
-  if (r.w == 0) return 0;
-  const int fa = max(b.time[b.out_src[e]], 0), fb = min(b.time[r.x], T);
-  *first = fa;
-  return fb > fa ? fb - fa : 0;
-}
-
 // One CTA per lattice: exclusive scan of the arcs' frame counts, then the
 // (frame, word) -> arc instances in arc order, each carrying the arc's TIME-ORDER index
-// (the stable sort then leaves every group in a fixed order).
+// (the stable sort then leaves every group in a fixed order).  Also the lattice of
+// each of the lattice's work items.
 __global__ void __launch_bounds__(256) k_fg_emit(GroupArgs a) {
   __shared__ int warp_sum[8];
   __shared__ int carry_s;
@@ -528,6 +525,7 @@ __global__ void __launch_bounds__(256) k_fg_emit(GroupArgs a) {
   const int T = b.fr_base[l + 1] - b.fr_base[l] - 1;
   const int64_t base = a.inst_base[l];
   const int tid = threadIdx.x;
+  for (int it = a.item_base[l] + tid; it < a.item_base[l + 1]; it += 256) a.item_lat[it] = l;
   if (tid == 0) carry_s = 0;
   __syncthreads();
   for (int tile = e0; tile < e1; tile += 256) {
@@ -547,15 +545,17 @@ __global__ void __launch_bounds__(256) k_fg_emit(GroupArgs a) {
   }
 }
 
-// one warp per run of frames.  WORDS == false: sorted instances -> frame_arc with head
-// bits, groups per frame.  WORDS == true (after the scans): the word of every group,
-// in output-row order.
+// one warp per run of frames.  WORDS == false: groups per frame and the run's window.
+// WORDS == true (after the scans and the window read back): the word and first instance
+// of every group, in output-row order, and every instance's offset in the run's window.
+// The run's instances are one contiguous range: the window and the offsets stream over it
+// with four loads in flight per lane, apart from the per-frame walk over the keys.
 template <bool WORDS>
 __global__ void __launch_bounds__(256) k_fg_heads(GroupArgs a) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const BatchView& b = a.b;
   for (int item = blockIdx.x * 8 + warp; item < a.num_items; item += gridDim.x * 8) {
-    const int l = last_le(a.item_base, 0, b.L - 1, item);
+    const int l = a.item_lat[item];
     const int T = b.fr_base[l + 1] - b.fr_base[l] - 1;
     const int k0 = (item - a.item_base[l]) * kFramesPerItem;
     const int k1 = min(T, k0 + kFramesPerItem);
@@ -563,7 +563,44 @@ __global__ void __launch_bounds__(256) k_fg_heads(GroupArgs a) {
     const unsigned int* key32 = reinterpret_cast<const unsigned int*>(key);
     const unsigned int* val = a.where[l] ? a.val_b : a.val_a;
     const unsigned long long label_mask = (1ULL << a.bits_label) - 1ULL;
-    int wlo = 0x7fffffff, whi = -1;  // arc id window of the run
+    const int64_t r0 = b.fr_off[b.fr_base[l] + k0], r1 = b.fr_off[b.fr_base[l] + k1];
+    if (!WORDS) {
+      int wlo = 0x7fffffff, whi = -1;  // arc id window of the run
+      for (int64_t i0 = r0 + lane; i0 < r1; i0 += 128) {
+        int e[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) e[u] = i0 + 32 * u < r1 ? (int)val[i0 + 32 * u] : -1;
+#pragma unroll
+        for (int u = 0; u < 4; ++u)
+          if (e[u] >= 0) {
+            wlo = min(wlo, e[u]);
+            whi = max(whi, e[u]);
+          }
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        wlo = min(wlo, __shfl_xor_sync(0xffffffffu, wlo, o));
+        whi = max(whi, __shfl_xor_sync(0xffffffffu, whi, o));
+      }
+      if (lane == 0) {
+        a.run_lo[item] = wlo;
+        a.run_hi[item] = whi;
+        if (whi >= wlo) atomicMax(a.max_window, whi - wlo + 1);
+      }
+    } else {
+      const unsigned int wlo = (unsigned int)a.run_lo[item];
+      for (int64_t i0 = r0 + lane; i0 < r1; i0 += 128) {
+        unsigned int id[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) id[u] = i0 + 32 * u < r1 ? val[i0 + 32 * u] - wlo : 0u;
+#pragma unroll
+        for (int u = 0; u < 4; ++u)
+          if (i0 + 32 * u < r1) {
+            if (a.id16) static_cast<uint16_t*>(a.ids)[i0 + 32 * u] = (uint16_t)id[u];
+            else static_cast<uint32_t*>(a.ids)[i0 + 32 * u] = id[u];
+          }
+      }
+    }
     for (int k = k0; k < k1; ++k) {
       const int fs = b.fr_base[l] + k;
       const int64_t f0 = b.fr_off[fs], f1 = b.fr_off[fs + 1];
@@ -577,14 +614,7 @@ __global__ void __launch_bounds__(256) k_fg_heads(GroupArgs a) {
           head = i == f0 || (a.k32 ? (unsigned long long)key32[i - 1] : key[i - 1]) != kk;
         }
         const unsigned int hm = __ballot_sync(0xffffffffu, head);
-        if (!WORDS) {
-          if (i < f1) {
-            const unsigned int e = val[i];
-            a.frame_arc[i] = (int32_t)(e | (head ? 0x80000000u : 0u));
-            wlo = min(wlo, (int)e);
-            whi = max(whi, (int)e);
-          }
-        } else if (head) {
+        if (WORDS && head) {
           const int64_t row = a.res_off[l] + a.gloc[fs] + groups + __popc(hm & ((1u << lane) - 1u));
           a.gwords[row] = (int32_t)(kk & label_mask);
           a.gframe[row] = k;
@@ -593,18 +623,6 @@ __global__ void __launch_bounds__(256) k_fg_heads(GroupArgs a) {
         groups += __popc(hm);
       }
       if (!WORDS && lane == 0) a.frame_cnt[fs] = groups;
-    }
-    if (!WORDS) {
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) {
-        wlo = min(wlo, __shfl_xor_sync(0xffffffffu, wlo, o));
-        whi = max(whi, __shfl_xor_sync(0xffffffffu, whi, o));
-      }
-      if (lane == 0) {
-        a.run_lo[item] = wlo;
-        a.run_hi[item] = whi;
-        if (whi >= wlo) atomicMax(a.max_window, whi - wlo + 1);
-      }
     }
   }
 }
@@ -639,12 +657,28 @@ int bits_for(int64_t maxv) {
 
 }  // namespace
 
-// Called by both packers once the packed arrays, state times and the frame CSR
-// offsets (fr_base, fr_off) are on the device.
+uint32_t frame_time_tail(int32_t max_time) {
+  // a word arc that spans a frame starts before its destination's time, so below max_time; the
+  // tail still fits the bits_for(max_time) bits the time order is sorted on
+  return (1u << bits_for(max_time)) - 1u;
+}
+
+int reserve_frame_time_keys(klu_ctx* c, uint32_t** keys) {
+  // build_frame_groups sorts the (frame, word) instances in the same buffer later: sized for both
+  const size_t n = std::max<size_t>((size_t)std::max<int64_t>(c->frame_entries, 0), (size_t)std::max<int64_t>(c->E, 1));
+  KLU_TRY(c->d_scratch[6].reserve(8 * n));
+  *keys = c->d_scratch[6].as<uint32_t>();
+  return 0;
+}
+
+// Called by both packers once the packed arrays, state times, the frame CSR offsets
+// (fr_base, fr_off) and the arcs' start-time keys (reserve_frame_time_keys) are on the device.
 int build_frame_groups(klu_ctx* c) {
   const int32_t L = c->L;
   c->h_frame_res_off.assign(L + 1, 0);
   c->fr_items = 0;
+  c->fr_max_window = 0;
+  c->fr_id16 = true;
   if (L == 0) return 0;
   bool any_bad_times = false;
   for (int32_t l = 0; l < L; ++l) any_bad_times |= !c->h_times_ok[l];
@@ -684,7 +718,7 @@ int build_frame_groups(klu_ctx* c) {
   }
   // scratch: the context's tool-scratch slots (free while loading; they stay allocated, so
   // repeated loads do not go through cudaMalloc / cudaFree again)
-  DevBuf &key_a = c->d_scratch[6], &key_b = c->d_scratch[7], &val_a = c->d_scratch[8], &val_b = c->d_scratch[9],
+  DevBuf &key_a = c->d_scratch[6] /* holds the start-time keys: see reserve_frame_time_keys */, &key_b = c->d_scratch[7], &val_a = c->d_scratch[8], &val_b = c->d_scratch[9],
          &misc = c->d_scratch[10];
   int rc = 0;
   do {
@@ -702,6 +736,7 @@ int build_frame_groups(klu_ctx* c) {
     if ((rc = small_h2d(c, d_inst_cnt, inst_cnt.data(), 4 * (size_t)L))) break;
     cudaMemsetAsync(d_frame_cnt, 0, 4 * (size_t)F, c->stream);
     if ((rc = c->d_frame_arc.reserve(4 * (size_t)N))) break;
+    if ((rc = c->d_fr_item_lat.reserve(4 * (size_t)std::max(c->fr_items, 1)))) break;
     GroupArgs a;
     a.b = c->view();
     a.bits_label = bits_label;
@@ -713,9 +748,11 @@ int build_frame_groups(klu_ctx* c) {
     a.val_a = val_a.as<unsigned int>();
     a.val_b = val_b.as<unsigned int>();
     a.where = d_where;
-    a.frame_arc = c->d_frame_arc.as<int32_t>();
+    a.ids = c->d_frame_arc.p;
+    a.id16 = 0;
     a.frame_cnt = d_frame_cnt;
     a.item_base = c->d_fr_item.as<int32_t>();
+    a.item_lat = c->d_fr_item_lat.as<int32_t>();
     a.num_items = c->fr_items;
     a.gloc = c->d_fr_gloc.as<int64_t>();
     a.lat_cnt = d_lat_cnt;
@@ -723,10 +760,10 @@ int build_frame_groups(klu_ctx* c) {
     //      one contiguous range of it), and the out-order -> time-order map for the instances
     {
       const size_t E1 = (size_t)std::max<int64_t>(c->E, 1);
-      if ((rc = key_a.reserve(8 * std::max<size_t>((size_t)N, E1))) || (rc = key_b.reserve(8 * std::max<size_t>((size_t)N, E1))) ||
+      uint32_t* tkeys = nullptr;  // already written: reserving again keeps them
+      if ((rc = reserve_frame_time_keys(c, &tkeys)) || (rc = key_b.reserve(8 * std::max<size_t>((size_t)N, E1))) ||
           (rc = val_a.reserve(4 * std::max<size_t>((size_t)N, E1))) || (rc = val_b.reserve(4 * std::max<size_t>((size_t)N, E1))) ||
-          (rc = c->d_scratch[11].reserve(4 * E1)) || (rc = c->d_fr_tarc.reserve(16 * E1)) ||
-          (rc = c->d_fr_tlabel.reserve(4 * E1)))
+          (rc = c->d_scratch[11].reserve(4 * E1)) || (rc = c->d_fr_tarc.reserve(16 * E1)))
         break;
       a.key = key_a.as<unsigned long long>();
       a.val = val_a.as<unsigned int>();
@@ -736,7 +773,6 @@ int build_frame_groups(klu_ctx* c) {
       a.val_b = val_b.as<unsigned int>();
       a.rank_of = c->d_scratch[11].as<int32_t>();
       a.tarc = c->d_fr_tarc.as<int4>();
-      a.tlabel = c->d_fr_tlabel.as<int32_t>();
       int64_t max_arcs = 0;
       std::vector<int64_t> arc_base(L + 1);
       std::vector<int32_t> arc_cnt(L);
@@ -844,6 +880,8 @@ int build_frame_groups(klu_ctx* c) {
     a.gwords = c->d_fr_gword.as<int32_t>();
     a.gframe = c->d_fr_gframe.as<int32_t>();
     a.gstart = c->d_fr_gstart.as<uint32_t>();
+    c->fr_id16 = c->fr_max_window < 65536;  // the layout k_frame_groups<Id> reads
+    a.id16 = c->fr_id16;
     {
       const uint32_t n32 = (uint32_t)N;
       if ((rc = small_h2d(c, a.gstart + c->h_frame_res_off[L], &n32, 4))) break;
@@ -886,6 +924,7 @@ int run_frame_post(klu_ctx* c, const klu_opts* o) {
   a.beta = c->d_beta.as<double>();
   a.total = c->d_total.as<double>();
   a.item_base = c->d_fr_item.as<int32_t>();
+  a.item_lat = c->d_fr_item_lat.as<int32_t>();
   a.num_items = c->fr_items;
   a.gloc = c->d_fr_gloc.as<int64_t>();
   a.res_off = c->d_fr_res_off.as<int64_t>();
@@ -896,15 +935,16 @@ int run_frame_post(klu_ctx* c, const klu_opts* o) {
   a.run_lo = c->d_fr_run_lo.as<int32_t>();
   a.run_hi = c->d_fr_run_hi.as<int32_t>();
   a.tarc = c->d_fr_tarc.as<int4>();
-  a.tlabel = c->d_fr_tlabel.as<int32_t>();
+  a.ids = c->d_frame_arc.p;
   if (a.num_items > 0) {
     // shared memory: the largest window of the batch, capped (runs beyond the cap take the slow path)
     const int kMaxWinBytes = 64 << 10;
-    KLU_CUDA(cudaFuncSetAttribute(k_frame_groups, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxWinBytes));  // per device
     const int kWinBytes = std::min(kMaxWinBytes, std::max(1024, (c->fr_max_window * 8 + 1023) & ~1023));
     a.win_cap = kWinBytes / 8;
+    auto* kern = c->fr_id16 ? k_frame_groups<uint16_t> : k_frame_groups<uint32_t>;
+    KLU_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxWinBytes));  // per device
     KLU_LAUNCH(c, "k_frame_groups");
-    k_frame_groups<<<a.num_items, 128, kWinBytes, c->stream>>>(a);
+    kern<<<a.num_items, 128, kWinBytes, c->stream>>>(a);
     KLU_TRY(check_launch("k_frame_groups"));
   }
   if (a.num_items > 0) {

@@ -51,7 +51,8 @@ struct GP {
   float *pfg, *pfa;
   int64_t *band_off, *fr_off;
   int4 *in_rec, *out_rec;
-  int32_t* frame_arc;
+  uint32_t* time_key;  // [E] the arcs' start-time keys of the frame index (reserve_frame_time_keys)
+  uint32_t time_tail;
   int32_t* counts;     // [S] scratch: per packed state count to be scanned
   int32_t* fr_cnt;     // per frame slot
   long long* lat_tot;  // [L+1] per-lattice totals / bases
@@ -389,7 +390,7 @@ __global__ void __launch_bounds__(256) k_gp_band_counts2(GP a) {
 
 // grid (L, tiles): +1 at the first frame of every word arc, -1 at the frame after its last one
 // (two atomics per arc, not one per arc x frame); k_gp_frame_counts turns the differences into the
-// arcs alive in every frame
+// arcs alive in every frame.  Also every arc's start-time key for build_frame_groups.
 __global__ void __launch_bounds__(256) k_gp_frames(GP a) {
   // (lattice-fastest grid on purpose: tile-fastest puts the CTAs in flight on the same few lattices'
   // frame counters and the atomics collide -- 5.8 vs 10.1 ms)
@@ -413,6 +414,7 @@ __global__ void __launch_bounds__(256) k_gp_frames(GP a) {
         }
       }
     }
+    if (p < e1) a.time_key[p] = fa >= 0 ? (uint32_t)fa : a.time_tail;
     const unsigned int ga = __match_any_sync(0xffffffffu, fa), gb = __match_any_sync(0xffffffffu, fb);
     if (fa >= 0 && lane == __ffs(ga) - 1) atomicAdd(cnt + fa, __popc(ga));
     if (fb >= 0 && lane == __ffs(gb) - 1) atomicAdd(cnt + fb, -__popc(gb));
@@ -871,8 +873,8 @@ int ensure_frame_index(klu_ctx* c) {
   const int st_tiles = (int)std::max<int64_t>(1, std::min<int64_t>((max_frames + 255) / 256, 16));
   KLU_TRY(stage_begin(c, (size_t)L));
   // ---- frame -> arc CSR ----
-  KLU_TRY(c->d_frame_arc.reserve(4 * (size_t)std::max<long long>(fa_base[L], 1)));
-  a.frame_arc = c->d_frame_arc.as<int32_t>();
+  KLU_TRY(reserve_frame_time_keys(c, &a.time_key));
+  a.time_tail = frame_time_tail(c->max_time);
   KLU_TRY(sc[R_VALB].reserve(4 * F1));  // frame counters (the sort buffers are free again)
   a.fr_cnt = sc[R_VALB].as<int32_t>();
   KLU_CUDA(cudaMemsetAsync(a.fr_cnt, 0, 4 * F1, c->stream));

@@ -291,16 +291,20 @@ int pack_and_upload(klu_ctx* c, const klu_lattices* in) {
     c->h_band_off.resize(L + 1);
     for (int32_t l = 0; l <= L; ++l) c->h_band_off[l] = st.band_off[in->state_off[l]];
   }
-  // frame -> arc CSR (the arc x frame expansion of latbin/lattice-to-word-frame-post.cc:110-116
-  // as an index structure): per lattice, per frame, the word arcs alive in it, in arc order
+  // frame -> arc CSR offsets (the arc x frame expansion of latbin/lattice-to-word-frame-post.cc:110-116
+  // as an index structure): per lattice, per frame, the first of the word arcs alive in it; and
+  // every arc's start-time key for build_frame_groups
   std::vector<int32_t> fr_base(L + 1, 0);
   std::vector<int64_t> fa_base(L + 1, 0);
+  int32_t max_time = 0;
   for (int32_t l = 0; l < L; ++l) {
     fr_base[l + 1] = fr_base[l] + info[l].num_frames + 1;
     fa_base[l + 1] = fa_base[l] + info[l].cap_frame;
+    max_time = std::max(max_time, std::max(info[l].max_time, info[l].num_frames));  // = c->max_time below
   }
   std::vector<int64_t> fr_off((size_t)fr_base[L] + 1, 0);
-  std::vector<int32_t> frame_arc((size_t)std::max<int64_t>(fa_base[L], 1));
+  const uint32_t time_tail = frame_time_tail(max_time);
+  std::vector<uint32_t> time_key((size_t)E, time_tail);
   {
     std::vector<std::thread> th;
     for (unsigned t = 0; t < nthreads; ++t)
@@ -316,15 +320,10 @@ int pack_and_upload(klu_ctx* c, const klu_lattices* in) {
             if (r.w == 0) continue;
             const int32_t fa = std::max(st.time[st.out_src[p]], 0), fb = std::min(st.time[r.x], T);
             for (int32_t k = fa; k < fb; ++k) cur[k + 1]++;
+            if (fb > fa) time_key[(size_t)p] = (uint32_t)fa;
           }
           for (int32_t k = 0; k < T; ++k) cur[k + 1] += cur[k];
           for (int32_t k = 0; k <= T; ++k) fo[k] = fa_base[l] + cur[k];
-          for (int64_t p = e0; p < e1; ++p) {
-            const int4 r = st.out_rec[p];
-            if (r.w == 0) continue;
-            const int32_t fa = std::max(st.time[st.out_src[p]], 0), fb = std::min(st.time[r.x], T);
-            for (int32_t k = fa; k < fb; ++k) frame_arc[(size_t)(fa_base[l] + cur[k]++)] = (int32_t)p;
-          }
         }
       });
     for (auto& x : th) x.join();
@@ -398,7 +397,11 @@ int pack_and_upload(klu_ctx* c, const klu_lattices* in) {
   KLU_TRY(up(c->d_order, st.order.data(), st.order.size() * 4));
   KLU_TRY(up(c->d_fr_base, fr_base.data(), fr_base.size() * 4));
   KLU_TRY(up(c->d_fr_off, fr_off.data(), fr_off.size() * 8));
-  KLU_TRY(up(c->d_frame_arc, frame_arc.data(), frame_arc.size() * 4));
+  {
+    uint32_t* keys = nullptr;
+    KLU_TRY(reserve_frame_time_keys(c, &keys));  // after c->frame_entries and c->E are set
+    if (E) KLU_CUDA(cudaMemcpyAsync(keys, time_key.data(), time_key.size() * 4, cudaMemcpyHostToDevice, c->stream));
+  }
   KLU_CUDA(cudaStreamSynchronize(c->stream));  // staging vectors die here
   return build_frame_groups(c);
 }
