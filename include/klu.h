@@ -18,10 +18,12 @@
  *                      (+ kwsbin2/utils.h:41-303, fstext/fstext-utils2.h:278-603)
  *   KLU_POSITION_POST  latbin/lattice-to-word-position-post.cc:70-141 (SURVEY.md 8f)
  *   KLU_CHAR_SEGMENT   kwsbin2/lattice-char-index-segment.cc:93-223 (SURVEY.md 8f)
- *                      (both char tools: the pseudo-word frontier is bounded by --nbest, see
+ *                      (all char tools: the pseudo-word frontier is bounded by --nbest, see
  *                      klu_opts.nbest)
  *   KLU_LENGTH_DIST    latbin/lattice-to-transcript-length-dist.cc:64-125 (SURVEY.md 8f)
  *   KLU_PRUNE_ARCS     latbin/lattice-prune-arcs.cc:34-84,136-165 (SURVEY.md 8f)
+ *   KLU_CHAR_UTTERANCE lattice-char-index-utterance (no reference binary; DESIGN.md section 7):
+ *                      per pseudo-word the probability that it occurs at least once in the line
  *
  * Plain pointers and sizes only; all pointers are HOST pointers.  Every function
  * returns 0 on success; on failure klu_last_error() (thread-local) explains.
@@ -61,7 +63,8 @@ enum klu_tool {
   KLU_POSITION_POST = 8,
   KLU_CHAR_SEGMENT = 9,
   KLU_LENGTH_DIST = 10,
-  KLU_PRUNE_ARCS = 11
+  KLU_PRUNE_ARCS = 11,
+  KLU_CHAR_UTTERANCE = 12
 };
 
 /* A batch of lattices as concatenated SoA arrays.  state_off/arc_off have
@@ -115,7 +118,9 @@ typedef struct klu_opts {
                        * not expanded (an exact cut: the rows and their order are those of the
                        * uncut search).  A lattice fails with "more than 2^24 trie nodes at one
                        * depth" only when nbest is not below its row count and its uncut frontier
-                       * is that large. */
+                       * is that large.  KLU_CHAR_UTTERANCE ranks by the occurrence probability,
+                       * computes it only for pseudo-words that can still reach the nbest best,
+                       * and breaks a tie at the cut by the smaller string. */
   /* char index label groups (kwsbin2/utils.h:41-84): parallel arrays label->group
    * (epsilon->0 and whitespace->1 included by the caller), the groups that
    * increment the word count (INT_MAX = default group, 2, 3, ...), and the
@@ -200,6 +205,9 @@ int klu_fetch_char_position(klu_ctx* ctx, int64_t* char_off, int32_t* chars, int
                             int32_t* t1, double* logp);
 /* char segment index (KLU_CHAR_SEGMENT): same layout, rows carry (t0, t1) only. */
 int klu_fetch_char_segment(klu_ctx* ctx, int64_t* char_off, int32_t* chars, int32_t* t0, int32_t* t1, double* logp);
+/* char utterance index (KLU_CHAR_UTTERANCE): same layout, rows carry logp = log P(the pseudo-word
+ * occurs at least once in the lattice) only, ordered by (logp desc, string asc). */
+int klu_fetch_char_utterance(klu_ctx* ctx, int64_t* char_off, int32_t* chars, double* logp);
 /* KLU_FWD_BWD / any run: per-state alpha, beta (input state numbering) and
  * per-lattice total = 0.5*(tot_fwd + beta[0]) */
 int klu_fetch_fwd_bwd(klu_ctx* ctx, double* alpha, double* beta, double* total);

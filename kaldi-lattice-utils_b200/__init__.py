@@ -12,7 +12,7 @@ import it through `__graft_entry__.load_package()` / importlib, e.g.
     spec.loader.exec_module(klu)
 """
 from . import binding, lattice, shard  # noqa: F401
-from .binding import (BEST_PATH2, CHAR_POSITION, CHAR_SEGMENT, FRAME_POST, LENGTH_DIST, FWD_BWD, POSITION, POSITION_POST, PRUNE_ARCS, PRUNE_DYN_BEAM,  # noqa: F401
+from .binding import (BEST_PATH2, CHAR_POSITION, CHAR_SEGMENT, CHAR_UTTERANCE, FRAME_POST, LENGTH_DIST, FWD_BWD, POSITION, POSITION_POST, PRUNE_ARCS, PRUNE_DYN_BEAM,  # noqa: F401
                       SEGMENT,
                       UTTERANCE, Engine, KluError)
 from .lattice import (Lattice, LatticeBatch, format_tuples, kaldi_float, make_lattice, read_text_ark,  # noqa: F401

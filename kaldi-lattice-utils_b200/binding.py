@@ -12,13 +12,14 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 
-SEGMENT, POSITION, UTTERANCE, FRAME_POST, PRUNE_DYN_BEAM, BEST_PATH2, CHAR_POSITION, FWD_BWD, POSITION_POST, CHAR_SEGMENT, LENGTH_DIST, PRUNE_ARCS = range(12)
+SEGMENT, POSITION, UTTERANCE, FRAME_POST, PRUNE_DYN_BEAM, BEST_PATH2, CHAR_POSITION, FWD_BWD, POSITION_POST, CHAR_SEGMENT, LENGTH_DIST, PRUNE_ARCS, CHAR_UTTERANCE = range(13)
 TOOL_NAMES = {SEGMENT: "lattice-word-index-segment", POSITION: "lattice-word-index-position",
               UTTERANCE: "lattice-word-index-utterance", FRAME_POST: "lattice-to-word-frame-post",
               PRUNE_DYN_BEAM: "lattice-prune-dyn-beam", BEST_PATH2: "lattice-best-path2",
               CHAR_POSITION: "lattice-char-index-position", FWD_BWD: "fwd-bwd",
               POSITION_POST: "lattice-to-word-position-post", CHAR_SEGMENT: "lattice-char-index-segment",
-              LENGTH_DIST: "lattice-to-transcript-length-dist", PRUNE_ARCS: "lattice-prune-arcs"}
+              LENGTH_DIST: "lattice-to-transcript-length-dist", PRUNE_ARCS: "lattice-prune-arcs",
+              CHAR_UTTERANCE: "lattice-char-index-utterance"}
 INT_MAX = 2**31 - 1
 
 # every symbol include/klu.h declares (checked by tests/test_capi_symbols.py)
@@ -26,6 +27,7 @@ SYMBOLS = ["klu_last_error", "klu_version", "klu_opts_default", "klu_device_coun
            "klu_host_alloc", "klu_host_free", "klu_topsort", "klu_load", "klu_run", "klu_sync", "klu_result_offsets",
            "klu_fetch_segment", "klu_fetch_position", "klu_fetch_utterance", "klu_fetch_frame_post", "klu_fetch_frame_post_csr", "klu_fetch_position_post", "klu_fetch_length_dist",
            "klu_fetch_best_path2", "klu_fetch_prune", "klu_result_char_sizes", "klu_fetch_char_position", "klu_fetch_char_segment",
+           "klu_fetch_char_utterance",
            "klu_fetch_fwd_bwd", "klu_timer_start", "klu_timer_stop", "klu_launch_count", "klu_profile_enable",
            "klu_profile_json", "klu_batch_stats", "klu_flush_l2", "klu_load_times"]
 
@@ -453,6 +455,22 @@ class Engine:
             res.append([("_".join(str(c) for c in chars[coff[i]:coff[i + 1]].tolist()), int(t0[i]), int(t1[i]),
                          float(lp[i])) for i in range(a, b)])
         return res
+
+    def char_utterance(self, wspace, other_groups=(), **o):
+        """lattice-char-index-utterance rows per lattice: (string, logp), logp = log P(the pseudo-word
+        occurs at least once in the line), ordered by (logp desc, string asc)."""
+        lg, inc, dele = char_groups(wspace, other_groups)
+        self.run(CHAR_UTTERANCE, label_group=lg, inc_groups=inc, del_groups=dele, **o)
+        off = self.offsets()
+        n = int(off[-1])
+        tot = C.c_int64()
+        _chk(self.L.klu_result_char_sizes(self.h, C.byref(tot)))
+        coff = np.zeros(n + 1, np.int64)
+        chars = np.zeros(tot.value, np.int32)
+        lp = np.zeros(n, np.float64)
+        _chk(self.L.klu_fetch_char_utterance(self.h, _p(coff), _p(chars), _p(lp)))
+        return [[("_".join(str(c) for c in chars[coff[i]:coff[i + 1]].tolist()), float(lp[i])) for i in range(a, b)]
+                for a, b in zip(off[:-1], off[1:])]
 
     # -- measurement ------------------------------------------------------------
     def timer_start(self):

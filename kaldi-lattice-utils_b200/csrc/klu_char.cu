@@ -347,6 +347,18 @@ struct Frontier {
 //      So U and a total differ from their exact values by < 2 * 2^31 * 2^-51 * M = 2^-19 M;
 //      delta = 2^-16 M is eight times that.  delta only keeps more, so it cannot change a result.
 // With nbest at least the rows a lattice ends up with, tau stays -inf and nothing is cut.
+// lattice-char-index-utterance runs the position frontier without counting groups (every split state
+// has count 0, so a trie node is one string and nd_total = log E[N(v)] + beta[start], N(v) = runs
+// spelling v on a path).  Its rows are the exact occurrence log-probabilities P(v) = P(N(v) >= 1)
+// (k_char_occ), and tau is the nbest-th best of those found so far:
+//   2'. P(v) <= E[N(v)] = exp(nd_total(v)) <= exp(U(p)) for every descendant v of p (step 2 needs no
+//       position or segment key), so the test of step 4 still never cuts a node that reaches tau.
+//   4'. k_char_occ computes P(v) only for final nodes with nd_total - beta[start] >= tau - delta; any
+//       other node is below the final tau by step 2', gets no value and is never a row.
+//   6'. The occurrence sum adds the same kinds of terms as nd_total and U: path costs (add) folded by
+//       log_add, over the same arcs and exits, each reaching the value through fewer than 2^31 steps
+//       (a DP cell is one of the batch's work items), so its rounding error obeys the same bound and
+//       delta covers the comparison of a rounded P(v) with a rounded U or nd_total.
 constexpr double kCutSlack = 1.0 / 65536.0;
 
 __device__ __forceinline__ bool below_cut(double ub_logp, double tau, double beta0) {
@@ -750,6 +762,193 @@ __global__ void __launch_bounds__(256) k_char_tile_scan(Frontier f) {
   if (tid == 0) f.ncnt[l] = carry_i;
 }
 
+// ---- 4b. lattice-char-index-utterance: exact occurrence probabilities ---------------------------
+// For a pseudo-word v (group gv, |v| = m) a first-occurrence DP over the split lattice (SURVEY.md
+// App. B.2 for characters), cells per state x:
+//   a0[x][g]   (g < NG) paths start -> x whose last arc has group g, that are not inside a run matching
+//              a prefix of v and have completed no occurrence of v;
+//   a[x][j]    (j = 1..m) the same inside a run of group gv whose labels so far spell v[0..j).
+// An arc x -> y of label c and group gy != g_x starts a run (to a[y][1] if gy = gv and c = v[0], else
+// to a0[y][gy]); when it leaves a[x][m] it completes an occurrence instead.  A same-group arc goes from
+// a[x][j] to a[x][j+1] if c = v[j], else to a0 (a run longer than v, or another string).  Completions
+// at x are the exit mass: P(v) = log-sum over x of a[x][m] + exit[x][gv].  Costs and beam tests are
+// those of the frontier.  Below the level where v's first character can be entered (the earliest state
+// of v's depth-0 ancestor) a0 = A and a = -inf; after the level of v's last item no completion is
+// possible: the DP runs over that level span only, a warp per node, its cells in a scratch chunk.
+//   PHASE 0: per item slot the scratch a node's DP needs (0 = no DP), the roots' first states, and the
+//            carried-over threshold keys (k_char_accum gathers none in this mode);
+//   PHASE 1: the DP of every slot with scratch, over the slots of a chunk of lattices; its value
+//            becomes the node's row value and goes to the threshold segment;
+//   PHASE 2: after the last depth, row values below the lattice's final tau are dropped (the rows
+//            left are the nbest best and whatever ties the nbest-th; the host breaks those ties).
+struct OccArgs {
+  double* nd_occ;              // per node: log-sum of the occurrence paths (row value), -inf = none
+  int32_t* nd_lo;              // per depth-0 node: its first item state
+  int32_t* need;               // per item slot: scratch doubles of its node's DP
+  const int32_t* loc;          // lattice-local exclusive scan of need
+  const int64_t* sbase;        // [L+1] first scratch double of each lattice
+  double* scratch;
+  int64_t chunk_base;          // scratch holds [chunk_base, chunk_base + capacity) of the batch
+  int64_t slot0, slot1;        // PHASE 1: item slots of the chunk
+  int64_t pool;                // PHASE 2: node pool slots in use
+  const int32_t* nd_lat;
+  unsigned long long* tasks;   // KLU_CHAR_DEBUG: DP tasks of this depth (else nullptr)
+};
+
+__device__ __forceinline__ int state_level(const CharArgs& a, int l, int s) {
+  const int* lv = a.b.lvl_start + a.b.lvl_off[l];
+  return last_le(lv, 0, a.b.lvl_off[l + 1] - a.b.lvl_off[l] - 1, s);
+}
+
+// level span [*j0, *j1] of node's DP (items [i, ...) of the current depth, first of the node)
+__device__ __forceinline__ void occ_span(const CharArgs& a, const Frontier& f, const OccArgs& q, int l, int64_t base,
+                                         int n, int i, int node, int* j0, int* j1) {
+  int root = node;
+  while (f.nd_parent[root] >= 0) root = f.nd_parent[root];
+  int k = i;
+  while (k + 1 < n && f.it_node[base + k + 1] == node) ++k;  // items are sorted by state: the last one is the latest
+  *j0 = state_level(a, l, q.nd_lo[root]);
+  *j1 = state_level(a, l, f.it_state[base + k]);
+}
+
+__device__ __forceinline__ double occ_a0(const CharArgs& a, int l, const double* sc, int s_lo, int W, int x, int g) {
+  if (x >= s_lo) return sc[(long long)(x - s_lo) * W + g];
+  if (a.nhi[x] < a.nlo[x]) return neg_inf();
+  return a.A[cell_of(a, l, x) + g];
+}
+
+template <int PHASE>
+__global__ void __launch_bounds__(256) k_char_occ(CharArgs a, Frontier f, OccArgs q) {
+  if (PHASE == 2) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < q.pool; i += (int64_t)gridDim.x * blockDim.x) {
+      const int l = q.nd_lat[i];
+      if (l < 0 || !(q.nd_occ[i] > neg_inf())) continue;
+      if (!(q.nd_occ[i] - a.beta[a.b.s_off[l]] >= f.tau[l])) q.nd_occ[i] = neg_inf();
+    }
+    return;
+  }
+  const int NG = a.NG;
+  if (PHASE == 0) {
+    const LatTile lt = lat_tile();
+    const int l = lt.l;
+    const int n = f.icnt[l];
+    const int64_t base = f.ibase[l];
+    const double beta0 = a.beta[a.b.s_off[l]];
+    const double tau = f.tau[l];
+    if (f.tk_cnt) {
+      const int keep = f.tk_keep[l];
+      const int64_t wb = f.tk_wbase[l], tb = f.tk_tbase[l];
+      for (int j = lt.tile * blockDim.x + threadIdx.x; j < keep; j += lt.tiles * blockDim.x) f.tk_work[wb + j] = f.tk_top[tb + j];
+    }
+    for (int i = lt.tile * blockDim.x + threadIdx.x; i < n; i += lt.tiles * blockDim.x) {
+      const int node = f.it_node[base + i];
+      int need = 0;
+      if (!(i > 0 && f.it_node[base + i - 1] == node)) {
+        q.nd_occ[node] = neg_inf();
+        if (f.depth == 0) q.nd_lo[node] = f.it_state[base + i];
+        const double total = f.nd_total[node];
+        if (total > neg_inf() && !below_cut(total - beta0, tau, beta0)) {
+          int j0, j1;
+          occ_span(a, f, q, l, base, n, i, node, &j0, &j1);
+          const int* lv = a.b.lvl_start + a.b.lvl_off[l];
+          const int m = f.nd_len[node];
+          need = (lv[j1 + 1] - lv[j0]) * (NG + m) + (m + 1) / 2;
+          if (q.tasks) atomicAdd(q.tasks, 1ULL);
+        }
+      }
+      q.need[base + i] = need;
+    }
+    return;
+  }
+  // PHASE 1: a warp per task; the warps of the grid take 32 slots at a time
+  const int lane = threadIdx.x & 31;
+  const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  const int64_t gw = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const BatchView& b = a.b;
+  for (int64_t s32 = q.slot0 + gw * 32; s32 < q.slot1; s32 += nwarps * 32) {
+    const int64_t s = s32 + lane;
+    unsigned int todo = __ballot_sync(0xffffffffu, s < q.slot1 && q.need[s] > 0);
+    while (todo) {
+      const int64_t slot = s32 + __ffs(todo) - 1;
+      todo &= todo - 1;
+      const int l = last_le(f.ibase, 0, b.L - 1, slot);
+      const int64_t base = f.ibase[l];
+      const int i = (int)(slot - base), n = f.icnt[l];
+      if (i >= n) continue;  // a slot past the lattice's items (PHASE 0 left its need unwritten)
+      const int node = f.it_node[slot];
+      const int g = f.nd_grp[node], m = f.nd_len[node], W = NG + m;
+      int j0, j1;
+      occ_span(a, f, q, l, base, n, i, node, &j0, &j1);
+      const int* lv = b.lvl_start + b.lvl_off[l];
+      const int s_lo = lv[j0];
+      double* sc = q.scratch + (q.sbase[l] + q.loc[slot] - q.chunk_base);
+      int* v = reinterpret_cast<int*>(sc + (long long)(lv[j1 + 1] - s_lo) * W);
+      if (lane == 0) {
+        int p = m, x = node;
+        while (x >= 0) {
+          v[--p] = f.nd_chr[x];
+          x = f.nd_parent[x];
+        }
+      }
+      __syncwarp();
+      double res = neg_inf();
+      for (int j = j0; j <= j1; ++j) {
+        const int y0 = lv[j], ny = lv[j + 1] - y0;
+        for (int c = lane; c < ny * W; c += 32) {
+          const int y = y0 + c / W, k = c % W;
+          double acc = neg_inf();
+          for (int e = b.in_off[y]; e < b.in_off[y + 1]; ++e) {
+            const int4 r = b.in_rec[e];
+            const int ge = group_of(a, r.w);
+            if (k < NG ? ge != k : (ge != g || r.w != v[k - NG])) continue;
+            const int x = r.x;
+            if (char_arc_pruned(a, l, x, y, r)) continue;
+            const double cost = rec_cost(r, a.cp);
+            if (k < NG) {
+              const bool first = k == g && r.w == v[0];  // a new run here matches v[0]
+              for (int gu = 0; gu < NG; ++gu) {
+                if (first && gu != k) continue;
+                const double xv = occ_a0(a, l, sc, s_lo, W, x, gu);
+                if (xv > neg_inf()) acc = log_add(acc, xv - cost);
+              }
+              if (x >= s_lo)
+                for (int jj = 1; jj <= m; ++jj) {
+                  if (k != g ? jj == m : (jj < m && r.w == v[jj])) continue;  // completed / matched on
+                  const double xv = sc[(long long)(x - s_lo) * W + NG + jj - 1];
+                  if (xv > neg_inf()) acc = log_add(acc, xv - cost);
+                }
+            } else if (k == NG) {  // a[y][1]: a run entered with v[0]
+              for (int gu = 0; gu < NG; ++gu) {
+                if (gu == g) continue;
+                const double xv = occ_a0(a, l, sc, s_lo, W, x, gu);
+                if (xv > neg_inf()) acc = log_add(acc, xv - cost);
+              }
+            } else if (x >= s_lo) {  // a[y][j], j >= 2
+              const double xv = sc[(long long)(x - s_lo) * W + k - 1];
+              if (xv > neg_inf()) acc = log_add(acc, xv - cost);
+            }
+          }
+          sc[(long long)(y - s_lo) * W + k] = acc;
+          if (k == W - 1 && acc > neg_inf()) {
+            const double ex = a.exitw[(long long)y * NG + g];
+            if (ex > neg_inf()) res = log_add(res, acc + ex);
+          }
+        }
+        __syncwarp();
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) res = log_add(res, __shfl_xor_sync(0xffffffffu, res, o));
+      if (lane == 0) {
+        q.nd_occ[node] = res;
+        const double logp = res - a.beta[b.s_off[l]];  // as k_char_rowkey forms it
+        if (f.tk_cnt && res > neg_inf() && logp > f.tau[l])
+          f.tk_work[f.tk_wbase[l] + atomicAdd(f.tk_cnt + l, 1)] = ~ord_f64(logp + 0.0);
+      }
+      __syncwarp();
+    }
+  }
+}
+
 // ---- 5. rows -----------------------------------------------------------------------
 struct RowArgs {
   int64_t pool;             // nodes in the pool
@@ -885,7 +1084,9 @@ CharState& char_state(klu_ctx* c) {
 
 }  // namespace
 
-int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
+// segment: lattice-char-index-segment keys (frame tags); utterance: lattice-char-index-utterance
+// (string keys, rows valued by k_char_occ); neither: lattice-char-index-position
+int run_char_index(klu_ctx* c, const klu_opts* o, bool segment, bool utterance) {
   const int32_t L = c->L;
   for (int32_t l = 0; l < L; ++l)
     if (!c->h_times_ok[l]) {
@@ -968,8 +1169,9 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
   a.dflt = dense(INT_MAX);
   a.eps = dense(0);
   a.segment = segment ? 1 : 0;
-  // the segment tool has no word-count split (kwsbin2/lattice-char-index-segment.cc:113-117)
-  for (int32_t i = 0; !segment && i < o->num_inc_groups; ++i) a.inc_mask |= 1u << dense(o->inc_groups[i]);
+  // the segment tool has no word-count split (kwsbin2/lattice-char-index-segment.cc:113-117), nor has
+  // the utterance tool (its keys are the strings alone)
+  for (int32_t i = 0; !segment && !utterance && i < o->num_inc_groups; ++i) a.inc_mask |= 1u << dense(o->inc_groups[i]);
   for (int32_t i = 0; i < o->num_del_groups; ++i) a.del_mask |= 1u << dense(o->del_groups[i]);
   a.use_beam = use_beam ? 1 : 0;
   a.vfwd = c->d_vfwd.as<double>();
@@ -1066,10 +1268,15 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
   KLU_TRY(cand_cnt.reserve(4 * E));
   KLU_TRY(cand_loc.reserve(4 * E));
   int64_t pool = 0;  // node pool slots in use
-  DevBuf* nd_all[11] = {&nd_parent, &nd_chr, &nd_cnt, &nd_grp, &nd_lat, &nd_t0, &nd_t1, &nd_len, &nd_total, &nd_best, &nd_ub};
+  // utterance: per node its row value and (depth 0) first state; per item slot the DP scratch it
+  // needs, its scan, the lattices' scratch bases, the scratch, the debug task count
+  DevBuf &nd_occ = buf(), &nd_lo = buf(), &occ_need = buf(), &occ_loc = buf(), &occ_base = buf(), &occ_scratch = buf(),
+         &d_tasks = buf();
+  DevBuf* nd_all[13] = {&nd_parent, &nd_chr, &nd_cnt, &nd_grp, &nd_lat, &nd_t0, &nd_t1, &nd_len, &nd_total, &nd_best, &nd_ub,
+                        &nd_occ, &nd_lo};
   auto grow_pool = [&](int64_t need) -> int {
-    for (int i = 0; i < 11; ++i) {
-      const size_t w = i >= 8 ? 8 : 4;
+    for (int i = 0; i < (utterance ? 13 : 11); ++i) {
+      const size_t w = (i >= 8 && i <= 11) ? 8 : 4;
       KLU_TRY(grow_keep(c, *nd_all[i], (size_t)pool * w, (size_t)need * w));
     }
     return 0;
@@ -1160,6 +1367,64 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
     KLU_TRY(check_launch("k_char_tau"));
     return 0;
   };
+  // utterance: the occurrence DPs of the nodes just folded (k_char_occ), in chunks of lattices whose
+  // scratch fits kOccChunk doubles
+  std::vector<int64_t> h_ibase(L + 1, 0);  // item slots of the current depth per lattice
+  OccArgs q;
+  memset(&q, 0, sizeof(q));
+  auto occ_depth = [&](int node_depth) -> int {
+    q.nd_occ = nd_occ.as<double>();
+    q.nd_lo = nd_lo.as<int32_t>();
+    KLU_TRY(occ_need.reserve(4 * (size_t)std::max<int64_t>(items_total, 1)));
+    KLU_TRY(occ_loc.reserve(4 * (size_t)std::max<int64_t>(items_total, 1)));
+    KLU_TRY(occ_base.reserve(8 * (size_t)(L + 1)));
+    q.need = occ_need.as<int32_t>();
+    q.loc = occ_loc.as<int32_t>();
+    q.sbase = occ_base.as<int64_t>();
+    q.tasks = nullptr;
+    if (debug) {
+      KLU_TRY(d_tasks.reserve(8));
+      KLU_CUDA(cudaMemsetAsync(d_tasks.p, 0, 8, c->stream));
+      q.tasks = d_tasks.as<unsigned long long>();
+    }
+    {
+      KLU_LAUNCH(c, "k_char_occ");
+      k_char_occ<0><<<dim3(L, 64), 256, 0, c->stream>>>(a, f, q);
+    }
+    KLU_TRY(check_launch("k_char_occ(count)"));
+    SegRange rg = {nullptr, f.ibase, f.icnt};
+    KLU_TRY(scan(rg, q.need, occ_loc.as<int32_t>(), occ_base.as<int64_t>()));
+    const std::vector<int64_t> sb = h_base;  // scratch doubles before each lattice
+    if (debug) {
+      unsigned long long h_tasks = 0;
+      KLU_CUDA(cudaMemcpyAsync(&h_tasks, d_tasks.p, 8, cudaMemcpyDeviceToHost, c->stream));
+      KLU_CUDA(cudaStreamSynchronize(c->stream));
+      fprintf(stderr, "[klu char] depth %d: %llu occurrence DP tasks, %lld scratch doubles\n", node_depth, h_tasks,
+              (long long)sb[L]);
+    }
+    q.tasks = nullptr;
+    constexpr int64_t kOccChunk = (int64_t)1 << 27;  // 1 GiB of scratch
+    for (int32_t l0 = 0; l0 < L;) {
+      int32_t l1 = l0 + 1;
+      while (l1 < L && sb[l1 + 1] - sb[l0] <= kOccChunk) ++l1;
+      const int64_t need = sb[l1] - sb[l0];
+      if (need > 0) {
+        KLU_TRY(occ_scratch.reserve(8 * (size_t)need));
+        q.scratch = occ_scratch.as<double>();
+        q.chunk_base = sb[l0];
+        q.slot0 = h_ibase[l0];
+        q.slot1 = h_ibase[l1];
+        const int64_t warps = std::max<int64_t>(1, (q.slot1 - q.slot0 + 31) / 32);
+        {
+          KLU_LAUNCH(c, "k_char_occ");
+          k_char_occ<1><<<(unsigned)std::min<int64_t>((warps + 7) / 8, (int64_t)c->num_sms * 8), 256, 0, c->stream>>>(a, f, q);
+        }
+        KLU_TRY(check_launch("k_char_occ"));
+      }
+      l0 = l1;
+    }
+    return 0;
+  };
   for (int depth = 0; depth < 100000; ++depth) {
     // ---- candidates: count, scan ----
     if (depth == 0) {
@@ -1182,10 +1447,13 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
         f.tk_cnt = tk_cnt.as<int32_t>();
       }
       {
+        Frontier g = f;
+        if (utterance) g.tk_cnt = nullptr;  // the threshold keys are the occurrence values (k_char_occ)
         KLU_LAUNCH(c, "k_char_accum");
-        k_char_accum<<<dim3(L, 64), 256, 0, c->stream>>>(a, f);
+        k_char_accum<<<dim3(L, 64), 256, 0, c->stream>>>(a, g);
       }
       KLU_TRY(check_launch("k_char_accum"));
+      if (utterance) KLU_TRY(occ_depth(depth - 1));
       if (nbest > 0) KLU_TRY(cut_update());
       if (debug) {
         KLU_CUDA(cudaMemsetAsync(d_cut.p, 0, 8, c->stream));
@@ -1362,8 +1630,20 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
     items_total = ncand;
     parent_pool_base = pool;
     pool += ncand;
+    if (utterance) h_ibase = h_base;
   }
   if (pool == 0) return 0;
+  if (utterance && nbest > 0) {  // rows: the nbest best occurrence values and their ties
+    q.pool = pool;
+    q.nd_lat = nd_lat.as<int32_t>();
+    q.nd_occ = nd_occ.as<double>();
+    {
+      KLU_LAUNCH(c, "k_char_occ");
+      k_char_occ<2><<<(unsigned)std::max<int64_t>(1, std::min<int64_t>((pool + 255) / 256, (int64_t)c->num_sms * 8)), 256, 0,
+                      c->stream>>>(a, f, q);
+    }
+    KLU_TRY(check_launch("k_char_occ(rows)"));
+  }
   // ---- rows ----
   DevBuf &row_cnt = buf(), &row_base = buf(), &cursor = buf(), &rkey_a = buf(), &rkey_b = buf(), &rval_a = buf(),
          &rval_b = buf(), &out_base = buf(), &o_node = buf(), &chr_off = buf();
@@ -1383,12 +1663,12 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
   r.nd_t0 = nd_t0.as<int32_t>();
   r.nd_t1 = nd_t1.as<int32_t>();
   r.nd_len = nd_len.as<int32_t>();
-  r.nd_total = nd_total.as<double>();
+  r.nd_total = utterance ? nd_occ.as<double>() : nd_total.as<double>();
   r.beta = a.beta;
   r.s_off = a.b.s_off;
   r.row_cnt = row_cnt.as<int32_t>();
   r.cursor = cursor.as<int32_t>();
-  r.nbest = o->nbest;
+  r.nbest = utterance ? INT_MAX : o->nbest;  // utterance: ties at the cut are broken on the host
   {
     KLU_LAUNCH(c, "k_char_rowcount");
     k_char_rowcount<<<c->num_sms * 4, 256, 0, c->stream>>>(r);
@@ -1400,7 +1680,7 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
   std::vector<int64_t> h_rbase(L + 1, 0), h_obase(L + 1, 0);
   for (int32_t l = 0; l < L; ++l) {
     h_rbase[l + 1] = h_rbase[l] + h_rows[l];
-    h_obase[l + 1] = h_obase[l] + std::min<int64_t>(h_rows[l], o->nbest);
+    h_obase[l + 1] = h_obase[l] + std::min<int64_t>(h_rows[l], r.nbest);
   }
   const int64_t nrows = h_rbase[L], nsel = h_obase[L];
   out.row_off = h_obase;
@@ -1522,7 +1802,9 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
   KLU_CUDA(cudaMemcpyAsync(out.chars.data(), c->d_res[6].p, 4 * (size_t)nchars, cudaMemcpyDeviceToHost, c->stream));
   KLU_CUDA(cudaStreamSynchronize(c->stream));
   // ---- final order of each lattice's rows (kwsbin2/lattice-char-index-position.cc:272-281):
-  //      logp desc, string asc (decimal labels joined by '_', compared as text), position asc
+  //      logp desc, string asc (decimal labels joined by '_', compared as text), position asc;
+  //      the utterance tool keeps the first nbest of that order (a tie at the cut goes to the
+  //      smaller string: its rows are the nbest best and everything tied with the nbest-th)
   {
     std::vector<std::string> str(nsel);
     for (int64_t i = 0; i < nsel; ++i) {
@@ -1544,25 +1826,32 @@ int run_char_index(klu_ctx* c, const klu_opts* o, bool segment) {
         return out.t1[x] < out.t1[y];
       });
     CharState s2;
-    s2.row_off = out.row_off;
+    s2.row_off.assign(L + 1, 0);
     s2.chr_off.assign(1, 0);
-    for (int64_t i = 0; i < nsel; ++i) {
-      const int64_t p = perm[i];
-      s2.pos.push_back(out.pos[p]);
-      s2.t0.push_back(out.t0[p]);
-      s2.t1.push_back(out.t1[p]);
-      s2.logp.push_back(out.logp[p]);
-      s2.chars.insert(s2.chars.end(), out.chars.begin() + out.chr_off[p], out.chars.begin() + out.chr_off[p + 1]);
-      s2.chr_off.push_back((int64_t)s2.chars.size());
+    for (int32_t l = 0; l < L; ++l) {
+      const int64_t end = std::min<int64_t>(h_obase[l + 1], h_obase[l] + std::max(o->nbest, 0));  // (utterance: the cut)
+      for (int64_t i = h_obase[l]; i < end; ++i) {
+        const int64_t p = perm[i];
+        s2.pos.push_back(out.pos[p]);
+        s2.t0.push_back(out.t0[p]);
+        s2.t1.push_back(out.t1[p]);
+        s2.logp.push_back(out.logp[p]);
+        s2.chars.insert(s2.chars.end(), out.chars.begin() + out.chr_off[p], out.chars.begin() + out.chr_off[p + 1]);
+        s2.chr_off.push_back((int64_t)s2.chars.size());
+      }
+      s2.row_off[l + 1] = (int64_t)s2.pos.size();
     }
     out = s2;
   }
+  c->h_res_off = out.row_off;
+  c->last_entries = out.row_off[L];
   c->last_chars = (int64_t)out.chars.size();
   return 0;
 }
 
-int run_char_position(klu_ctx* c, const klu_opts* o) { return run_char_index(c, o, false); }
-int run_char_segment(klu_ctx* c, const klu_opts* o) { return run_char_index(c, o, true); }
+int run_char_position(klu_ctx* c, const klu_opts* o) { return run_char_index(c, o, false, false); }
+int run_char_segment(klu_ctx* c, const klu_opts* o) { return run_char_index(c, o, true, false); }
+int run_char_utterance(klu_ctx* c, const klu_opts* o) { return run_char_index(c, o, false, true); }
 
 void char_release(klu_ctx* c) {
   delete static_cast<CharState*>(c->char_state);
@@ -1577,7 +1866,7 @@ using namespace klu;
 extern "C" {
 
 int klu_result_char_sizes(klu_ctx* c, int64_t* total_chars) {
-  if (c->last_tool != KLU_CHAR_POSITION && c->last_tool != KLU_CHAR_SEGMENT) {
+  if (c->last_tool != KLU_CHAR_POSITION && c->last_tool != KLU_CHAR_SEGMENT && c->last_tool != KLU_CHAR_UTTERANCE) {
     set_error("klu_result_char_sizes: last run was not a char index tool");
     return 1;
   }
@@ -1614,6 +1903,17 @@ int klu_fetch_char_segment(klu_ctx* c, int64_t* char_off, int32_t* chars, int32_
   c->last_tool = KLU_CHAR_POSITION;  // same row store
   const int rc = klu_fetch_char_position(c, char_off, chars, nullptr, t0, t1, logp);
   c->last_tool = KLU_CHAR_SEGMENT;
+  return rc;
+}
+
+int klu_fetch_char_utterance(klu_ctx* c, int64_t* char_off, int32_t* chars, double* logp) {
+  if (c->last_tool != KLU_CHAR_UTTERANCE) {
+    set_error("klu_fetch_char_utterance: last run was not KLU_CHAR_UTTERANCE");
+    return 1;
+  }
+  c->last_tool = KLU_CHAR_POSITION;  // same row store
+  const int rc = klu_fetch_char_position(c, char_off, chars, nullptr, nullptr, nullptr, logp);
+  c->last_tool = KLU_CHAR_UTTERANCE;
   return rc;
 }
 

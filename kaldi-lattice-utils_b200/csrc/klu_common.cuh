@@ -240,6 +240,7 @@ int run_length_dist(klu_ctx* c, const klu_opts* o);
 // klu_char.cu
 int run_char_position(klu_ctx* c, const klu_opts* o);
 int run_char_segment(klu_ctx* c, const klu_opts* o);
+int run_char_utterance(klu_ctx* c, const klu_opts* o);
 void char_release(klu_ctx* c);
 
 CostParams make_cost_params(const klu_opts* o, bool float_sum);

@@ -498,6 +498,9 @@ int klu_run(klu_ctx* c, int tool, const klu_opts* opts) {
     case KLU_CHAR_SEGMENT:
       rc = run_char_segment(c, opts);
       break;
+    case KLU_CHAR_UTTERANCE:
+      rc = run_char_utterance(c, opts);
+      break;
     case KLU_LENGTH_DIST:
       rc = run_length_dist(c, opts);
       break;

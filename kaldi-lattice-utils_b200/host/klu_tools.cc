@@ -14,6 +14,7 @@
 //   lattice-to-word-position-post latbin/lattice-to-word-position-post.cc:28-147 (SURVEY.md 8f)
 //   lattice-char-index-segment    kwsbin2/lattice-char-index-segment.cc:249-349 (SURVEY.md 8f)
 //   lattice-to-transcript-length-dist latbin/lattice-to-transcript-length-dist.cc:28-131 (SURVEY.md 8f)
+//   lattice-char-index-utterance  (no reference binary; the flags of lattice-char-index-segment)
 //
 // Lattices are independent, so the reader fills a batch (KLU_BATCH_ARCS arcs,
 // default 32M), the batch is packed/uploaded/processed, and entries are written
@@ -53,7 +54,7 @@ namespace {
 
 // The tools close a batch at this many lattices whatever their size (archives of tiny lattices:
 // bounds the per-lattice host metadata of a batch); the library itself has no such limit.
-#if KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */
+#if KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */ || KLU_TOOL == 12 /* KLU_CHAR_UTTERANCE */
 // The character tools keep every same-group sub-path of a batch in device memory at once (a trie
 // whose frontier can grow by the branching factor per character): small batches bound that
 // (256 c5 lattices: ~1.6e8 candidates at the deepest level, a few GB).
@@ -251,6 +252,12 @@ void ComputeBatch(klu_ctx* ctx, const klu_opts* opts, const Batch* b, Results* r
     r->coff.resize(n + 1), r->chars.resize((size_t)total_chars);
     r->i2.resize(n), r->i3.resize(n), r->d0.resize(n);
     KLU_CHECK(klu_fetch_char_segment(ctx, r->coff.data(), r->chars.data(), r->i2.data(), r->i3.data(), r->d0.data()));
+#elif KLU_TOOL == 12 /* KLU_CHAR_UTTERANCE */
+    int64_t total_chars = 0;
+    KLU_CHECK(klu_result_char_sizes(ctx, &total_chars));
+    r->coff.resize(n + 1), r->chars.resize((size_t)total_chars);
+    r->d0.resize(n);
+    KLU_CHECK(klu_fetch_char_utterance(ctx, r->coff.data(), r->chars.data(), r->d0.data()));
 #elif KLU_TOOL == 3 /* KLU_FRAME_POST */
     // rows without the per-row frame column (a third of the download); the writer below shares
     // its loop with the position-post / length-dist tools, which carry one, so it is rebuilt here
@@ -354,7 +361,7 @@ void EmitBatch(ToolState* st, Batch* b, Results* r) {
     if (!bin) os << '\n';
     w.End();
   }
-#elif KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */
+#elif KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */ || KLU_TOOL == 12 /* KLU_CHAR_UTTERANCE */
   for (int32_t l = 0; l < L; ++l) {
     std::ostream& os = w.Begin(b->lats[l].key);
     const size_t a = (size_t)off[l], e = (size_t)off[l + 1];
@@ -373,8 +380,10 @@ void EmitBatch(ToolState* st, Batch* b, Results* r) {
 #if KLU_TOOL == 6 /* KLU_CHAR_POSITION */
       WriteBasicInt32(os, bin, r->i1[i]);
 #endif
+#if KLU_TOOL != 12 /* KLU_CHAR_UTTERANCE: (string, logp) */
       WriteBasicInt32(os, bin, r->i2[i]);
       WriteBasicInt32(os, bin, r->i3[i]);
+#endif
       WriteBasicDouble(os, bin, r->d0[i]);
       WriteTupleSep(os, bin, i - a, e - a);
     }
@@ -643,7 +652,7 @@ int main(int argc, char* argv[]) {
   // heap (no mmap / munmap and fresh page faults per array)
   mallopt(M_MMAP_THRESHOLD, 1 << 30);
   mallopt(M_TRIM_THRESHOLD, 1 << 30);
-#if KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */
+#if KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */ || KLU_TOOL == 12 /* KLU_CHAR_UTTERANCE */
   const int kErrorCode = 1;  // kwsbin2/lattice-char-index-position.cc:405-408
 #else
   const int kErrorCode = -1;  // e.g. kwsbin2/lattice-word-index-position.cc:293-296
@@ -689,6 +698,13 @@ int main(int argc, char* argv[]) {
         "optional other groups, default group) and every maximal sub-path of same-group arcs is a pseudo-word.\n\n"
         "Usage: lattice-char-index-segment [options] separator-symbols lat-rspecifier index-wspecifier\n"
         " e.g.: lattice-char-index-segment \"3 4\" ark:1.lats ark:1.index\n";
+#elif KLU_TOOL == 12 /* KLU_CHAR_UTTERANCE */
+    const char* usage =
+        "Build an utterance-level word index from character lattices: the score of each pseudo-word is the "
+        "probability that it occurs at least once in the line. Characters are grouped (whitespace group, optional "
+        "other groups, default group) and every maximal sub-path of same-group arcs is a pseudo-word.\n\n"
+        "Usage: lattice-char-index-utterance [options] separator-symbols lat-rspecifier index-wspecifier\n"
+        " e.g.: lattice-char-index-utterance \"3 4\" ark:1.lats ark:1.index\n";
 #elif KLU_TOOL == 3 /* KLU_FRAME_POST */
     const char* usage =
         "Compute the posterior log-probability of each word for each given utterance frame. That is, we compute "
@@ -727,7 +743,7 @@ int main(int argc, char* argv[]) {
     po.Register("insertion-penalty", &insertion_penalty,
                 "Add this penalty to the lattice arcs with non-epsilon output label (typically, equivalent to word "
                 "insertion penalty).");
-#if KLU_TOOL == 1 /* KLU_POSITION */ || KLU_TOOL == 0 /* KLU_SEGMENT */ || KLU_TOOL == 2 /* KLU_UTTERANCE */ || KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */
+#if KLU_TOOL == 1 /* KLU_POSITION */ || KLU_TOOL == 0 /* KLU_SEGMENT */ || KLU_TOOL == 2 /* KLU_UTTERANCE */ || KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */ || KLU_TOOL == 12 /* KLU_CHAR_UTTERANCE */
     po.Register("beam", &beam, "Pruning beam (applied after acoustic scaling and adding the insertion penalty).");
     po.Register("num-threads", &num_threads, "Accepted for compatibility; lattices are batched on the GPU instead.");
     po.Register("num-threads-total", &num_threads_total, "Accepted for compatibility; ignored.");
@@ -742,7 +758,7 @@ int main(int argc, char* argv[]) {
     int32_t rho_label = INT_MAX;
     po.Register("rho-label", &rho_label, "Accepted for compatibility (no composition is materialised).");
 #endif
-#if KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */
+#if KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */ || KLU_TOOL == 12 /* KLU_CHAR_UTTERANCE */
     float determinize_delta = 1.0f / 1024.0f / 8.0f;
     po.Register("nbest", &st.opts.nbest, "Extract this number of n-best hypothesis.");
     po.Register("determinize-delta", &determinize_delta,
@@ -762,7 +778,7 @@ int main(int argc, char* argv[]) {
 #endif
     po.Read(argc, argv);
 
-#if KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */
+#if KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */ || KLU_TOOL == 12 /* KLU_CHAR_UTTERANCE */
     if (po.NumArgs() != 3) {
       po.PrintUsage();
       exit(1);
@@ -817,7 +833,7 @@ int main(int argc, char* argv[]) {
     st.opts.num_include = (int32_t)st.include.size();
     st.opts.exclude_words = st.exclude.data();
     st.opts.num_exclude = (int32_t)st.exclude.size();
-#if KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */
+#if KLU_TOOL == 6 /* KLU_CHAR_POSITION */ || KLU_TOOL == 9 /* KLU_CHAR_SEGMENT */ || KLU_TOOL == 12 /* KLU_CHAR_UTTERANCE */
     {
       // kwsbin2/utils.h:41-84 ParseSeparatorGroups
       std::map<int32_t, int32_t> label_group;
